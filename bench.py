@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: tets/s of fwd+bwd G-Shell / mSDF extraction (BASELINE.json metric) + HBM roofline fraction.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -26,6 +26,7 @@ import subprocess
 import sys
 import threading
 import time
+import zlib
 
 import numpy as np
 
@@ -70,7 +71,10 @@ def parse():
                          "ranges are sharded over the ranks + NCCL all-gather of the valid-tet records")
     ap.add_argument("--frames-total", type=int, default=16, help="--mode strong: frames per step over ALL ranks")
     ap.add_argument("--blocks", type=int, default=5,
-                    help="the timed block of --steps steps is repeated this many times; value = median block")
+                    help="the --steps timed steps are split into this many blocks run back to back; value = median block")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (rank 0's frames: surfaces, counts, "
+                         "gradients) as DIR/<name>.npy, float32 / float64, at most 64 MB in all")
     ap.add_argument("--api", default="packed", choices=["packed", "frames"],
                     help="batch results as padded (B,cap,..) tensors (O(1) host work per batch) or as per-frame tuples")
     ap.add_argument("--no-cold", action="store_true", help="skip the L2-flushed single-call leg")
@@ -117,6 +121,12 @@ def make_config(args, world, F, N, counts0, ngroups, frames_per_step):
                   % (34 * max(1, frames_per_step // max(world, 1))),
             "lanes": args.lanes, "groups": ngroups, "mode": args.mode,
             "parallelism": (("frames x%d" % world) if args.mode != "tets" else ("tet ranges x%d" % world)) if world > 1 else "single GPU"}
+
+
+def block_sizes(steps, blocks):
+    """Exactly `steps` timed steps, split into up to `blocks` blocks that run back to back."""
+    n = max(1, min(blocks, steps))
+    return [(b + 1) * steps // n - b * steps // n for b in range(n)]
 
 
 def group_bounds(n, groups):
@@ -172,6 +182,53 @@ class ClockSampler(threading.Thread):
             return {"sm_mhz": None, "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons), "samples": 0}
         return {"sm_mhz": float(np.median(self.samples)), "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons),
                 "samples": len(self.samples)}
+
+
+# ------------------------------------------------------------------------------------------------- --dump-outputs
+DUMP_LIMIT = 64 << 20
+#: the gradients on the grid are almost all zero; they are kept on the grid vertices nearest the surface (smallest
+#: |sdf|), where the rows the extraction touches lie
+DUMP_GRID_ROWS = 1 << 16
+SURFACE_OUTPUTS = ("verts_aug", "faces_aug", "v_tng_aug", "msdf", "vertices_watertight", "faces_watertight",
+                   "v_tng_watertight", "msdf_watertight")
+
+
+def step_outputs(groups, flat_grad, rows):
+    """What a caller of the timed step holds afterwards, as numpy.  `groups`: (results, gradient of the positions) of
+    every extract_frames_async call of the step, results packed or per frame.  Per frame, concatenated over the frames
+    in order: the reference's outputs and `counts` (rows of verts_aug, faces_aug, vertices_watertight and
+    faces_watertight).  The gradients of pos (frame-major), sdf and msdf on the grid vertices `rows`."""
+    per, counts, g_pos = {k: [] for k in SURFACE_OUTPUTS}, [], []
+    for res, g in groups:
+        frames = [res.frame(i) for i in range(len(res))] if hasattr(res, "frame") else res
+        for verts, faces, _, _, v_tng, extra in frames:
+            vals = (verts, faces, v_tng, extra["msdf"], extra["vertices_watertight"], extra["faces_watertight"],
+                    extra["v_tng_watertight"], extra["msdf_watertight"])
+            for k, t in zip(SURFACE_OUTPUTS, vals):
+                per[k].append(t.detach().cpu().numpy())
+            counts.append([vals[i].shape[0] for i in (0, 1, 4, 5)])
+        g_pos.append(g[:, rows].reshape(-1, 3).cpu().numpy())
+    n = flat_grad.shape[0] // 2
+    out = {k: np.concatenate(v) for k, v in per.items()}
+    out.update(counts=np.array(counts), grad_pos=np.concatenate(g_pos), grad_sdf=flat_grad[:n][rows].cpu().numpy(),
+               grad_msdf=flat_grad[n:][rows].cpu().numpy())
+    return out
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT):
+    """Writes every array as out_dir/<name>.npy: float32 stays float32, anything else becomes float64 (exact for the
+    integer outputs).  An array larger than an equal share of `limit` keeps a sample of its rows, drawn with a seed of
+    its own and sorted, so that two runs with the same row count keep the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = (limit - 4096 * len(arrays)) // len(arrays)      # 4096: room for the .npy header
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        a = a.astype(np.float32 if a.dtype == np.float32 else np.float64, copy=False)
+        if a.nbytes > share:
+            keep = np.random.default_rng(zlib.crc32(name.encode())).choice(a.shape[0], share // (a.nbytes // a.shape[0]),
+                                                                            replace=False)
+            a = a[np.sort(keep)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------- reference arm
@@ -310,10 +367,9 @@ def run_tets(args, rank, local_rank, world, dev, dev_type):
         step()
     sampler = ClockSampler(local_rank)
     sampler.start()
-    steps = min(args.steps, 50)
     l0 = E.launch_counter()
-    blocks = [timed(steps) for _ in range(max(1, args.blocks))]
-    launches = (E.launch_counter() - l0) // max(1, args.blocks)
+    blocks = [timed(n) for n in block_sizes(args.steps, args.blocks)]
+    launches = E.launch_counter() - l0
     sampler.stop_flag = True
     sampler.join(timeout=2)
     ms = float(np.median(blocks))
@@ -332,7 +388,7 @@ def run_tets(args, rank, local_rank, world, dev, dev_type):
         except Exception:
             pass
         balg = grids.surface_counts_bytes(F, N, c0["n_verts"], c0["n_verts_aug"], c0["n_faces_watertight"], c0["n_faces_aug"])
-        line = {"metric": METRIC, "value": F / (ms * 1e-3), "unit": UNIT, "n_gpus": world, "steps": steps,
+        line = {"metric": METRIC, "value": F / (ms * 1e-3), "unit": UNIT, "n_gpus": world, "steps": args.steps,
                 "warmup": max(args.warmup, 3), "ms_per_step": ms, "higher_is_better": True, "scaling": "strong",
                 "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": tets_config(args, world, F, N, c0),
                 "ms_per_step_blocks": [round(b, 5) for b in blocks],
@@ -351,6 +407,8 @@ def main():
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs and (args.impl == "reference" or args.mode == "tets"):
+        raise SystemExit("--dump-outputs: only the batched extraction (--impl ours, --mode weak / strong) keeps its outputs")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
@@ -427,6 +485,7 @@ def main():
         for i in range(lo, hi):
             pups_v[k][i - lo, :ups_v[i].shape[0]] = ups_v[i]
             pups_m[k][i - lo, :ups_m[i].shape[0]] = ups_m[i]
+    last_step = []      # --dump-outputs: (results, gradient of the positions) of every group of the latest step
 
     def local_step():
         """This rank's share of a step, no collective: every group of frames is one extract_frames_async call (one
@@ -436,17 +495,20 @@ def main():
         sdf.grad, msdf.grad = flat_grad[:N].view(N, 1), flat_grad[N:]
         for pg in pos_groups:
             pg.grad = None
+        last_step.clear()
         futs = [E.extract_frames_async(pg, sdf, msdf, tets, types="cloth", lanes=args.lanes) for pg in pos_groups]
         for k, (fut, (lo, hi)) in enumerate(zip(futs, gb)):
             if args.api == "packed":
-                pk = fut.packed()
+                res = pk = fut.packed()
                 cva = pk.verts_aug.shape[1]
                 if cva > pad_rows:
                     raise RuntimeError("bench: padded upstream gradients too small for the plan's capacity")
                 torch.autograd.backward([pk.verts_aug, pk.msdf], [pups_v[k][:, :cva], pups_m[k][:, :cva]])
             else:
-                outs = fut.result()
+                res = outs = fut.result()
                 torch.autograd.backward([o[0] for o in outs] + [o[5]["msdf"] for o in outs], ups_v[lo:hi] + ups_m[lo:hi])
+            if args.dump_outputs:
+                last_step.append((res, pos_groups[k].grad))
 
     def step():
         """One training-step's worth of extraction: local_step() + the sum of the shared gradients over the ranks (ONE
@@ -487,16 +549,18 @@ def main():
         step()
     sampler = ClockSampler(local_rank)
     sampler.start()
-    # the timed block (exactly --steps steps between two barriers, CUDA events, max over ranks) is repeated --blocks
-    # times back to back; the reported time is the MEDIAN block (one block is tens of ms: a single one is at the mercy
-    # of a clock ramp or a host hiccup)
-    block_ms, launches_timed = [], 0
-    for _ in range(max(1, args.blocks)):
-        launches0 = E.launch_counter()
-        block_ms.append(timed(step, args.steps))
-        launches_timed = E.launch_counter() - launches0  # library kernels enqueued by this rank in one timed block
+    # exactly --steps timed steps in up to --blocks blocks run back to back (each between two barriers, CUDA events, max
+    # over ranks); the reported time is the MEDIAN block (one block is tens of ms: a single one is at the mercy of a clock
+    # ramp or a host hiccup)
+    launches0 = E.launch_counter()
+    block_ms = [timed(step, n) for n in block_sizes(args.steps, args.blocks)]
+    launches_timed = E.launch_counter() - launches0      # library kernels enqueued by this rank in the timed steps
     ms_step = float(np.median(block_ms))
     value = fps * F / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        rows = torch.from_numpy(np.sort(np.argsort(np.abs(sdf_np), kind="stable")[:DUMP_GRID_ROWS])).to(dev)
+        dump_outputs(args.dump_outputs, step_outputs(last_step, flat_grad, rows))
+    last_step.clear()
 
     # ---- where a step's time goes on every rank: the local part (no collective) and the exchange alone ----
     ranks_info = None

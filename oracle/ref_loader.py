@@ -1,10 +1,11 @@
 """Loader for the LIVE reference extraction classes (test infrastructure only).
 
-Reads `geometry/gshell_tets.py` / `geometry/hmsdf_tets_split.py` from the read-only reference tree at run
-time (nothing is copied into this repo), swaps the hard-coded 'cuda' device literals for the requested
+Reads `geometry/gshell_tets.py` / `geometry/hmsdf_tets_split.py` from a checkout of the original D3Human-code
+project at run time (nothing is copied into this repo), swaps the hard-coded 'cuda' device literals for the requested
 device (the reference hard-codes device='cuda' 19 times, e.g. gshell_tets.py:108) and stubs the two imports
-of render/util.py:12-13 that the extraction path never uses.  Only available in the build container:
-`/root/reference` does not exist on the GPU box, so everything that runs there uses the committed goldens.
+of render/util.py:12-13 that the extraction path never uses.  The checkout is not part of this repository: point
+D3H_REFERENCE_ROOT at it to run the live-reference tests; without it they skip and the committed goldens (written from
+the original by oracle/make_golden*.py) stand in for it.
 """
 from __future__ import annotations
 
@@ -12,11 +13,11 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("D3H_REFERENCE_ROOT", "/root/reference")
+REF_ROOT = os.environ.get("D3H_REFERENCE_ROOT", "")
 
 
 def reference_available() -> bool:
-    return os.path.isfile(os.path.join(REF_ROOT, "geometry", "gshell_tets.py"))
+    return bool(REF_ROOT) and os.path.isfile(os.path.join(REF_ROOT, "geometry", "gshell_tets.py"))
 
 
 def load_reference_class(which: str = "GShell_Tets", device: str = "cpu"):

@@ -12,4 +12,4 @@ warnings.filterwarnings("ignore", message=".*torch.cross.*")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs the live reference tree at /root/reference")
+    config.addinivalue_line("markers", "reference: needs a checkout of the original project (D3H_REFERENCE_ROOT)")

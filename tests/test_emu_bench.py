@@ -74,7 +74,7 @@ def _worker(rank, world, port, out_dir, argv):
 def test_bench_control_flow(tmp_path, world):
     import torch.multiprocessing as mp
     argv = ["--gpus", str(world), "--steps", "2", "--warmup", "1", "--res", "6", "--frames-per-rank", "16", "--groups", "2",
-            "--lanes", "2", "--profile-steps", "1", "--e2e-chunk", "8"]
+            "--lanes", "2", "--profile-steps", "1", "--e2e-chunk", "8", "--dump-outputs", str(tmp_path / "dump")]
     if world > 1:
         argv.append("--no-cpu-baseline")     # N = 1 runs the CPU baseline leg as well (tiny grid: a fraction of a second)
     ctx = mp.start_processes(_worker, args=(world, _free_port(), str(tmp_path), argv), nprocs=world, join=False,
@@ -107,7 +107,8 @@ def test_bench_control_flow(tmp_path, world):
         assert d["mesh_stage"] is None and d["torch_gpu_baseline"] is None
     for r in range(1, world):                    # only rank 0 prints
         assert not [l for l in open(tmp_path / f"out_{r}.txt") if l.startswith("{")]
-    assert len(d["ms_per_step_blocks"]) == 5 and d["config"]["mode"] == "weak"
+    assert len(d["ms_per_step_blocks"]) == 2 and d["config"]["mode"] == "weak"       # --steps 2: two blocks of one step
+    _check_dump(tmp_path / "dump", world)
     rk = d["ranks"]
     assert len(rk["local_step_ms"]) == world and rk["frames"] == [16] * world and all(t > 0 for t in rk["local_step_ms"])
     assert (world == 1) == (sum(rk["allreduce_ms"]) == 0)
@@ -117,6 +118,64 @@ def test_bench_control_flow(tmp_path, world):
         assert "error" not in sp and sp["two_calls_ms"] > 0 and sp["split_ms"] > 0 and sp["split_fused_ms"] > 0, sp
         # the compact gradient return: far fewer bytes back than the dense (N,3) gradients it replaces
         assert d["e2e"]["d2h_bytes_per_step"] < d["e2e"]["h2d_bytes_per_step"] * 4
+
+
+def _check_dump(out_dir, world):
+    """--dump-outputs of test_bench_control_flow (res 6, 16 frames on rank 0, nothing sampled at this size): the surfaces
+    of every frame are the oracle's; on one rank the gradients are the oracle's adjoint of bench.py's upstream gradients."""
+    import numpy as np
+    from oracle import gshell_oracle as O
+    from d3human_code_b200 import grids
+    from tests import _util as U
+    sys.path.insert(0, ROOT)
+    import bench
+    got = {n: np.load(out_dir / f"{n}.npy") for n in bench.SURFACE_OUTPUTS + ("counts", "grad_pos", "grad_sdf", "grad_msdf")}
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())
+    pos, sdf, msdf, tets = bench.make_inputs(6, "capsule")
+    N = pos.shape[0]
+    want = {n: [] for n in got}
+    gen = torch.Generator(device="cpu").manual_seed(1234)
+    fwds = [O.extract_forward(pos + grids.frame_offsets(N, 6, f), sdf, msdf, tets, 1, True) for f in range(16)]
+    ups_v = [torch.randn(fw["verts_aug"].shape, generator=gen).numpy() for fw in fwds]
+    ups_m = [torch.randn(fw["msdf"].shape, generator=gen).numpy() for fw in fwds]
+    want["grad_sdf"], want["grad_msdf"] = np.zeros(N), np.zeros(N)
+    for fw, gv, gm in zip(fwds, ups_v, ups_m):
+        for n in bench.SURFACE_OUTPUTS:
+            want[n].append(fw[n])
+        want["counts"].append([len(fw["verts_aug"]), len(fw["faces_aug"]), len(fw["vertices_watertight"]),
+                               len(fw["faces_watertight"])])
+        g_pos, g_sdf, g_msdf = O.extract_backward(fw, gv, gm)
+        want["grad_pos"].append(g_pos)
+        want["grad_sdf"] += g_sdf
+        want["grad_msdf"] += g_msdf
+    for n in bench.SURFACE_OUTPUTS:
+        w = np.concatenate(want[n])
+        if n.startswith("v_tng"):          # sums of float atomics in any order, as everywhere against the oracle
+            U.assert_tangents_close(n, got[n], w, U.TNG_CUDA_ATOL)
+        else:
+            assert got[n].shape == w.shape and np.array_equal(got[n], w), n
+    assert np.array_equal(got["counts"], np.array(want["counts"]))
+    assert got["grad_pos"].shape == (16 * N, 3) and got["grad_sdf"].shape == got["grad_msdf"].shape == (N,)
+    if world == 1:
+        for n in ("grad_pos", "grad_sdf", "grad_msdf"):
+            w = np.concatenate(want[n]) if n == "grad_pos" else want[n]
+            assert np.abs(got[n] - w).max() <= 1e-4 * np.abs(w).max(), n
+
+
+def test_dump_outputs_keeps_a_fixed_sample_of_large_arrays(tmp_path):
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    big = np.random.default_rng(0).standard_normal((5000, 3)).astype(np.float32)
+    arrays = {"small": np.arange(12, dtype=np.int32).reshape(4, 3), "big": big}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays, limit=64 << 10)
+    small, kept = np.load(tmp_path / "a" / "small.npy"), np.load(tmp_path / "a" / "big.npy")
+    assert small.dtype == np.float64 and np.array_equal(small, arrays["small"])
+    assert kept.dtype == np.float32 and 1000 < kept.shape[0] and kept.nbytes <= (64 << 10) // 2
+    assert np.array_equal(kept, np.load(tmp_path / "b" / "big.npy"))        # the same rows every run
+    rows = [int(np.flatnonzero((big == r).all(1))[0]) for r in kept]
+    assert rows == sorted(set(rows))                                          # rows of the array, in order
 
 
 def _run(tmp_path, world, argv, timeout=240):

@@ -56,7 +56,7 @@ def reference_lbs(pts, template, w, init_a, a, trans, grads=None):
 @pytest.mark.parametrize("seed", range(4))
 def test_oracle_matches_reference_methods(seed):
     if not ref_loader.reference_available():
-        pytest.skip("needs /root/reference")
+        pytest.skip("needs a checkout of the original project (D3H_REFERENCE_ROOT)")
     template, w, init_a, a, trans = synthetic_rig(seed)
     rng = np.random.default_rng(100 + seed)
     pts = rng.uniform(-1.1, 1.1, size=(700, 3)).astype(np.float32)

@@ -39,7 +39,7 @@ def test_oracle_reproduces_golden_vectors(path):
 
 def test_layer_shapes_match_the_reference_module():
     if not ref_loader.reference_available():
-        pytest.skip("needs /root/reference")
+        pytest.skip("needs a checkout of the original project (D3H_REFERENCE_ROOT)")
     import torch
     ref = ref_loader.load_reference_mlp()
     for cfg in (dict(n_freq=6, d_hidden=256, n_hidden=6, skip_in=[3]), dict(), dict(n_freq=3, d_hidden=32, n_hidden=2, skip_in=[0, 1])):
@@ -51,7 +51,7 @@ def test_layer_shapes_match_the_reference_module():
 @pytest.mark.parametrize("seed", range(6))
 def test_oracle_matches_live_reference(seed):
     if not ref_loader.reference_available():
-        pytest.skip("needs /root/reference")
+        pytest.skip("needs a checkout of the original project (D3H_REFERENCE_ROOT)")
     import torch
     ref = ref_loader.load_reference_mlp()
     rng = np.random.default_rng(seed)
