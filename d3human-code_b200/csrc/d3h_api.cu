@@ -168,6 +168,7 @@ Workspace carve_workspace(void* base, int64_t n_tets, int64_t n_grid, int64_t ca
   ws.poly_excl = reinterpret_cast<unsigned*>(take((ws.ntiles_poly + 1) * 32));
   // ... and per 32-polygon group (one warp of poly_faces_kernel): 8 words per group
   ws.poly_gcnt = reinterpret_cast<unsigned*>(take((ws.ntiles_poly + 1) * (kPolyThreads / 32) * 32));
+  ws.poly_used = reinterpret_cast<unsigned char*>(take(cap));
   ws.vert = reinterpret_cast<float4*>(take(capc * 16));
   ws.acc = reinterpret_cast<float*>(take(capc * 32));
   ws.owner = reinterpret_cast<int32_t*>(take(capc * 4));

@@ -68,6 +68,7 @@ struct Workspace {
   unsigned* poly_cnt;             // ntiles_poly * 8: polygons per faces_aug bucket in each polygon tile
   unsigned* poly_excl;            // ntiles_poly * 8: exclusive prefix of poly_cnt over the tiles
   unsigned* poly_gcnt;            // ntiles_poly * 8 * 8: the same counts per group of 32 polygons
+  unsigned char* poly_used;       // cap_valid_tets: per polygon, the boundary vertices its mSDF cut references (bit k: edge k -> k+1)
   float4* vert;                   // (x,y,z,msdf) per watertight vertex, 4*cap_valid_tets
   float* acc;                     // 8 floats per watertight vertex: normal xyz + count, tangent xyz + pad
   int32_t* owner;                 // per watertight vertex: the polygon corner slot that writes its tangent rows
@@ -97,7 +98,8 @@ __device__ __forceinline__ void shift_workspace(Workspace& w, int64_t shift) {
   D3H_SHIFT(mocc_bits); D3H_SHIFT(m1_words); D3H_SHIFT(m2_words); D3H_SHIFT(tile_cnt); D3H_SHIFT(records); D3H_SHIFT(keys);
   D3H_SHIFT(vals); D3H_SHIFT(keys2); D3H_SHIFT(vals2); D3H_SHIFT(keys_scratch); D3H_SHIFT(vals_scratch); D3H_SHIFT(msd_hist);
   D3H_SHIFT(msd_fill); D3H_SHIFT(msd_base); D3H_SHIFT(st_scan); D3H_SHIFT(group_start); D3H_SHIFT(group_heads);
-  D3H_SHIFT(gblock_heads); D3H_SHIFT(poly_cnt); D3H_SHIFT(poly_excl); D3H_SHIFT(poly_gcnt); D3H_SHIFT(vert); D3H_SHIFT(acc);
+  D3H_SHIFT(gblock_heads); D3H_SHIFT(poly_cnt); D3H_SHIFT(poly_excl); D3H_SHIFT(poly_gcnt); D3H_SHIFT(poly_used);
+  D3H_SHIFT(vert); D3H_SHIFT(acc);
   D3H_SHIFT(owner); D3H_SHIFT(edge_bits); D3H_SHIFT(word_prefix); D3H_SHIFT(eblock_cnt); D3H_SHIFT(corner_rank);
   D3H_SHIFT(q_cnt); D3H_SHIFT(vlist); D3H_SHIFT(elist); D3H_SHIFT(elist2); D3H_SHIFT(tet_word_prefix);
 #undef D3H_SHIFT

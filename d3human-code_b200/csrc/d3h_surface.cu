@@ -62,61 +62,136 @@ __device__ __forceinline__ int cut_case(bool quad, float m0, float m1, float m2,
   return ncut ? (ncut - 1) : -1;
 }
 
+// poly_cut_kernel: four lanes per polygon (lane k = corner k; the fourth lane of a triangle polygon idles): a 256-thread
+// CTA takes 64 polygons = two of poly_faces_kernel's 32-polygon groups.  Every lane evaluates ONE vertex frame and ONE
+// boundary vertex and writes at most one cut triangle; the values of the neighbouring corner travel by warp shuffles.
+// (v1 gave a whole polygon to one thread: four vertex frames in sequence on 226 CTAs, 14 us for 58 k polygons.)
+constexpr int kCutPolysPerCta = kPolyThreads / 4;
+
+// cut tables as shared-memory words (the case code differs from lane to lane: __constant__ would serialise)
+struct CutTables {
+  unsigned long long quad[16];   // 12 locals x 4 bits
+  unsigned tri[8];               //  6 locals x 4 bits
+  unsigned char nq[16], nt[8];   // number of cut triangles
+  unsigned char uq[16], ut[8];   // locals referenced by the cut triangles (bit mask)
+};
+
+__device__ __forceinline__ void load_cut_tables(CutTables& T) {
+  const unsigned t = threadIdx.x;
+  if (t < 16u) {
+    unsigned long long w = 0ull;
+    unsigned used = 0u;
+    const int n = c_num_cut_quad[t];
+    for (int e = 0; e < 12; ++e) {
+      const int loc = c_cut_quad[t][e];
+      w |= (unsigned long long)(loc & 0xf) << (4 * e);
+      if (e < 3 * n) used |= 1u << loc;
+    }
+    T.quad[t] = w; T.nq[t] = (unsigned char)n; T.uq[t] = (unsigned char)used;
+  } else if (t < 24u) {
+    const unsigned c = t - 16u;
+    unsigned w = 0u, used = 0u;
+    const int n = c_num_cut_tri[c];
+    for (int e = 0; e < 6; ++e) {
+      const int loc = c_cut_tri[c][e];
+      w |= (unsigned)(loc & 0xf) << (4 * e);
+      if (e < 3 * n) used |= 1u << loc;
+    }
+    T.tri[c] = w; T.nt[c] = (unsigned char)n; T.ut[c] = (unsigned char)used;
+  }
+}
+
+// what the topology CTAs of poly_cut_kernel write for one frame
+struct CutOut {
+  int64_t* faces_aug;
+  float* verts_aug;
+  float* msdf_aug;
+  int64_t cap_faces_aug, cap_verts_aug;
+};
+
 // REPLAY = second extraction of a cloth / body pair (d3h_forward_args.pair_*): `blk` is the pair's argument block (its
 // outputs, the opposite msdf_negate), the interpolated mSDF of every vertex is the exact negation of the stored one,
 // normals / tangents were accumulated by the first extraction and are not splatted again.
+//
+// Both surface kernels have two kinds of CTAs.  Frames that share sdf and msdf share one topology (BatchCtx), and all of
+// a polygon that follows from its corner ids and the interpolated mSDF alone -- the corner ids on the tape, the watertight
+// faces, the mSDF cut case, the rank in its faces_aug bucket, the faces_aug rows, the boundary mSDF -- is the same for each
+// of them.  CTAs [0, topo_ctas) of a row are TOPOLOGY CTAs: they do that work once per topology and store the result into
+// every frame of the launch that uses it.  When all `topo_rows` rows of the launch share one topology they split its tiles
+// (row r takes tiles [r * topo_ctas, (r + 1) * topo_ctas)); otherwise topo_rows = 1 and every row does its own.  The
+// other CTAs of a row are the frame's own and do only what needs its positions: normals, tangents, boundary vertices.
 // resident CTAs per SM the compiler has to leave room for (register cap): A/B by -D at build time
 #ifndef D3H_FACES_MINB
 #define D3H_FACES_MINB 4   // 64 registers instead of 80
 #endif
 #ifndef D3H_CUT_MINB
-#define D3H_CUT_MINB 4     // 62 registers (5 would be 48 + a 28-byte spill)
+#define D3H_CUT_MINB 5     // 48 registers, no spill: five CTAs per SM (4 allows 49 and leaves four)
 #endif
+
+// vertex id of a corner on the static edge table paths = number of marked edges before its edge in the static edge list
+__device__ __forceinline__ int edge_vertex(const unsigned* __restrict__ edge_bits, const unsigned* __restrict__ word_prefix,
+                                           unsigned r) {
+  return (int)(__ldcg(word_prefix + (r >> 5)) + __popc(__ldcg(edge_bits + (r >> 5)) & ((1u << (r & 31u)) - 1u)));
+}
+
+// corner ids of a polygon: on the tape ([3*T1 | 4*T2], gshell_tets.py:406-407), or from the static edge ranks
+__device__ __forceinline__ void polygon_corners(bool static_edges, const int32_t* __restrict__ corners,
+                                                const unsigned* __restrict__ corner_rank, const unsigned* __restrict__ edge_bits,
+                                                const unsigned* __restrict__ word_prefix, int64_t i, int64_t p0, int n,
+                                                int (&L)[4]) {
+  if (static_edges) {
+    const uint4 rk = __ldcg(reinterpret_cast<const uint4*>(corner_rank) + i);
+    const unsigned rr[4] = {rk.x, rk.y, rk.z, rk.w};
+#pragma unroll
+    for (int k = 0; k < 4; ++k) L[k] = (k < n) ? edge_vertex(edge_bits, word_prefix, rr[k]) : 0;
+  } else {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) L[k] = (k < n) ? corners[p0 + k] : 0;
+  }
+}
+
+// the watertight triangle t of a polygon: its corners in face order (select without dynamic register indexing)
+template <typename T>
+__device__ __forceinline__ void triangle_corners(int code, int t, const T (&in)[4], T (&out)[3]) {
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    const int lp = pos_in_loop(code, c_tri_edge[code][3 * t + c]);
+    out[c] = lp == 0 ? in[0] : lp == 1 ? in[1] : lp == 2 ? in[2] : in[3];
+  }
+}
+
 template <bool REPLAY>
 __global__ void __launch_bounds__(kPolyThreads, D3H_FACES_MINB)
 poly_faces_kernel(const FwdBlock* __restrict__ blk, const d3h_tet_record* __restrict__ records,
                   DevCounters* __restrict__ ctr, const float4* __restrict__ w_vert, float* __restrict__ w_acc,
                   unsigned* __restrict__ poly_cnt, unsigned* __restrict__ poly_gcnt, unsigned* __restrict__ poly_excl,
-                  UvParams uvp,
+                  unsigned char* __restrict__ poly_used, UvParams uvp,
                   d3h_counts* __restrict__ counts_dev, const unsigned* __restrict__ corner_rank,
-                  const unsigned* __restrict__ edge_bits, const unsigned* __restrict__ word_prefix, const __grid_constant__ FrameSet fs,
-                  const __grid_constant__ FrameSet topo) {
+                  const unsigned* __restrict__ edge_bits, const unsigned* __restrict__ word_prefix, unsigned topo_ctas,
+                  unsigned topo_rows, const __grid_constant__ FrameSet fs, const __grid_constant__ FrameSet topo) {
   pdl_enter();
-  // frames that share their topology (BatchCtx): the records and the corner ids were made once, by the first frame of the
-  // launch; this frame reads them there and leaves a copy of the corner ids on its own tape (poly_cut_kernel, backward)
-  const int32_t* __restrict__ corners_src = frame_ptr(blk, topo.off[blockIdx.y])->a.tape_corners;
-  {
-    const int64_t shift = fs.off[blockIdx.y];
-    records = frame_ptr(records, topo.off[blockIdx.y]);
-    blk = frame_ptr(blk, shift); ctr = frame_ptr(ctr, shift);
-    w_vert = frame_ptr(w_vert, shift); w_acc = frame_ptr(w_acc, shift); poly_cnt = frame_ptr(poly_cnt, shift);
-    poly_gcnt = frame_ptr(poly_gcnt, shift); poly_excl = frame_ptr(poly_excl, shift); counts_dev = frame_ptr(counts_dev, shift);
-    corner_rank = frame_ptr(corner_rank, shift); edge_bits = frame_ptr(edge_bits, shift);
-    word_prefix = frame_ptr(word_prefix, shift);
-  }
   constexpr int WARPS = kPolyThreads / 32;
-  int32_t* __restrict__ corners = blk->a.tape_corners;
+  const int64_t shift = fs.off[blockIdx.y], tshift = topo.off[blockIdx.y];
+  // the topology: records, corner ids (on the tape of its frame) and static edge ranks
+  records = frame_ptr(records, tshift);
+  corner_rank = frame_ptr(corner_rank, tshift); edge_bits = frame_ptr(edge_bits, tshift);
+  word_prefix = frame_ptr(word_prefix, tshift);
+  const FwdBlock* __restrict__ tblk = frame_ptr(blk, tshift);
+  int32_t* __restrict__ corners = tblk->a.tape_corners;
   // a replay finds the corner array on the tape, and so does the edge-scan path (scan_emit_kernel wrote it)
-  const bool static_edges = !REPLAY && blk->a.edge_off != nullptr && blk->a.etets == nullptr;
-  int64_t* __restrict__ faces_wt = blk->a.faces_wt;
-  const int64_t cap_faces_wt = blk->a.cap_faces_wt;
-  __shared__ unsigned s_cnt[8][WARPS];
-  __shared__ unsigned s_last;
-  __shared__ unsigned long long s_scan[3][32];
-
-  const unsigned t1 = ctr->work_tri, t2 = ctr->work_quad;
-  unsigned long long* tr = trace_begin(ctr->trace, ctr->trace_frame, K_POLY_FACES);
-  const int64_t npoly = (int64_t)t1 + t2;
-  const int64_t ntiles = (npoly + kPolyThreads - 1) / kPolyThreads;
-  const unsigned tile = blockIdx.x;
-  // CTAs past the data still take part in the "last CTA out" count (the grid is sized from the capacity)
+  const bool static_edges = !REPLAY && tblk->a.edge_off != nullptr && tblk->a.etets == nullptr;
   const unsigned lane = lane_id(), warp = threadIdx.x >> 5;
-  const int64_t i = (int64_t)tile * kPolyThreads + threadIdx.x;
-  const int64_t n_faces_total = (int64_t)t1 + 2ll * t2;
-  const bool cross_quirk = (n_faces_total == 3);  // torch.cross without dim on a (3,3) tensor, gshell_tets.py:19
 
-  if ((int64_t)tile < ntiles) {
-    int bucket = -1;
+  if (blockIdx.x >= topo_ctas) {
+    // ---- the frame's own CTAs: face normals / tangents of its positions, splatted to the watertight vertices ----
+    if (REPLAY) return;   // (not launched: normals / tangents were accumulated by the first extraction of the pair)
+    const DevCounters* __restrict__ fc = frame_ptr(ctr, shift);
+    w_vert = frame_ptr(w_vert, shift); w_acc = frame_ptr(w_acc, shift);
+    const unsigned t1 = fc->work_tri, t2 = fc->work_quad;
+    unsigned long long* tr = trace_begin(fc->trace, fc->trace_frame, K_POLY_FACES);
+    const int64_t npoly = (int64_t)t1 + t2;
+    const int64_t i = (int64_t)(blockIdx.x - topo_ctas) * kPolyThreads + threadIdx.x;
+    const bool cross_quirk = ((int64_t)t1 + 2ll * t2 == 3);  // torch.cross without dim on a (3,3) tensor, gshell_tets.py:19
     if (i < npoly) {
       const int4 meta = reinterpret_cast<const int4*>(records + i)[1];
       const int code = meta.x, rank = meta.y;
@@ -125,52 +200,15 @@ poly_faces_kernel(const FwdBlock* __restrict__ blk, const d3h_tet_record* __rest
       const int64_t p0 = quad ? (3ll * t1 + 4ll * rank) : 3ll * rank;
       int L[4];
       float4 P[4];
-      if (static_edges) {
-        // vertex id of a corner = number of marked edges before its edge in the static edge list; the corner array of
-        // the tape ([3*T1 | 4*T2], gshell_tets.py:406-407) is written here for poly_cut_kernel and the backward pass
-        const uint4 rk = __ldcg(reinterpret_cast<const uint4*>(corner_rank) + i);
-        const unsigned rr[4] = {rk.x, rk.y, rk.z, rk.w};
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          L[k] = 0;
-          if (k < n) {
-            const unsigned r = rr[k];
-            L[k] = (int)(__ldcg(word_prefix + (r >> 5)) + __popc(__ldcg(edge_bits + (r >> 5)) & ((1u << (r & 31u)) - 1u)));
-            corners[p0 + k] = L[k];
-          }
-        }
-      } else {
-#pragma unroll
-        for (int k = 0; k < 4; ++k) L[k] = (k < n) ? corners_src[p0 + k] : 0;
-        if (corners_src != corners) {
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            if (k < n) corners[p0 + k] = L[k];
-        }
-      }
+      polygon_corners(static_edges, corners, corner_rank, edge_bits, word_prefix, i, p0, n, L);
 #pragma unroll
       for (int k = 0; k < 4; ++k) P[k] = (k < n) ? w_vert[L[k]] : make_float4(0.f, 0.f, 0.f, 0.f);
-      // ---- watertight faces + splats ----
       const int ntri = quad ? 2 : 1;
       for (int t = 0; t < ntri; ++t) {
-        const int64_t row = quad ? ((int64_t)t1 + 2ll * rank + t) : (int64_t)rank;
-        int lp[3];
-#pragma unroll
-        for (int c = 0; c < 3; ++c) lp[c] = pos_in_loop(code, c_tri_edge[code][3 * t + c]);
-        // select without dynamic register indexing
         int vi[3];
         float4 pv[3];
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-          vi[c] = lp[c] == 0 ? L[0] : lp[c] == 1 ? L[1] : lp[c] == 2 ? L[2] : L[3];
-          pv[c] = lp[c] == 0 ? P[0] : lp[c] == 1 ? P[1] : lp[c] == 2 ? P[2] : P[3];
-        }
-        if (row < cap_faces_wt) {
-          faces_wt[3 * row + 0] = vi[0];
-          faces_wt[3 * row + 1] = vi[1];
-          faces_wt[3 * row + 2] = vi[2];
-        }
-        if (REPLAY) continue;  // normals / tangents were accumulated by the first extraction of the pair
+        triangle_corners(code, t, L, vi);
+        triangle_corners(code, t, P, pv);
         const float ax = __fsub_rn(pv[1].x, pv[0].x), ay = __fsub_rn(pv[1].y, pv[0].y), az = __fsub_rn(pv[1].z, pv[0].z);
         const float bx = __fsub_rn(pv[2].x, pv[0].x), by = __fsub_rn(pv[2].y, pv[0].y), bz = __fsub_rn(pv[2].z, pv[0].z);
         // accumulator row of a vertex: [nx ny nz count | tx ty tz -]; one 16-byte vector atomic per half (sm_90+)
@@ -196,32 +234,9 @@ poly_faces_kernel(const FwdBlock* __restrict__ blk, const d3h_tet_record* __rest
         for (int c = 0; c < 3; ++c)
           atomicAdd(reinterpret_cast<float4*>(w_acc + 8ll * vi[c]) + 1, make_float4(tx, ty, tz, 0.f));
       }
-      unsigned mcase;
-      int ncut;
-      const float sg = REPLAY ? -1.f : 1.f;  // exact: the pair's interpolated mSDF is the negation (SURVEY A.4)
-      bucket = cut_case(quad, sg * P[0].w, sg * P[1].w, sg * P[2].w, sg * P[3].w, mcase, ncut);
-    }
-    // ---- polygons per bucket: per group of 32 polygons (one warp; poly_cut_kernel ranks inside a tile with them) and
-    // per tile of 256 (scanned below by the last CTA).  Lane b keeps the count of bucket b ----
-    unsigned mine = 0u;
-#pragma unroll
-    for (int b = 0; b < 6; ++b) {
-      const unsigned m = __ballot_sync(0xffffffffu, bucket == b);
-      if (lane == (unsigned)b) mine = __popc(m);
-    }
-    if (lane < 8u) {   // (entries 6, 7: zero)
-      poly_gcnt[((int64_t)tile * WARPS + warp) * 8 + lane] = mine;
-      s_cnt[lane][warp] = mine;
-    }
-    __syncthreads();
-    if (threadIdx.x < 8) {
-      unsigned run = 0;
-#pragma unroll
-      for (int w = 0; w < WARPS; ++w) run += s_cnt[threadIdx.x][w];
-      poly_cnt[(int64_t)tile * 8 + threadIdx.x] = run;
     }
     // the (3,3) torch.cross quirk: the three face normals are crossed along the *face* axis
-    if (!REPLAY && cross_quirk && i == 0) {
+    if (cross_quirk && i == 0) {
       float a[3][3], b[3][3];
       int fv[3][3];
       for (int64_t q = 0; q < npoly; ++q) {
@@ -234,12 +249,7 @@ poly_faces_kernel(const FwdBlock* __restrict__ blk, const d3h_tet_record* __rest
           float4 pv[3];
           for (int c = 0; c < 3; ++c) {
             const int kk = pos_in_loop(code, c_tri_edge[code][3 * t + c]);
-            if (static_edges) {
-              const unsigned r = __ldcg(corner_rank + 4 * q + kk);
-              fv[row][c] = (int)(__ldcg(word_prefix + (r >> 5)) + __popc(__ldcg(edge_bits + (r >> 5)) & ((1u << (r & 31u)) - 1u)));
-            } else {
-              fv[row][c] = corners[p0 + kk];
-            }
+            fv[row][c] = static_edges ? edge_vertex(edge_bits, word_prefix, __ldcg(corner_rank + 4 * q + kk)) : corners[p0 + kk];
             pv[c] = w_vert[fv[row][c]];
           }
           a[row][0] = __fsub_rn(pv[1].x, pv[0].x); a[row][1] = __fsub_rn(pv[1].y, pv[0].y); a[row][2] = __fsub_rn(pv[1].z, pv[0].z);
@@ -255,13 +265,117 @@ poly_faces_kernel(const FwdBlock* __restrict__ blk, const d3h_tet_record* __rest
           for (int k = 0; k < 3; ++k) atomicAdd(w_acc + 8ll * fv[r][k] + c, fn[r]);  // counts were added above
       }
     }
+    if (tr != nullptr) __syncthreads();
+    trace_end(tr);
+    return;
   }
 
-  // ---- last CTA out: scan the tile counts, finalise and publish the sizes of this call ----
+  // ---- topology CTAs: corner ids and watertight faces of every frame, mSDF cut case and the polygons per faces_aug
+  // bucket of every group and tile (poly_cut_kernel ranks with them); the last one out scans the tiles and publishes ----
+  DevCounters* __restrict__ tc = frame_ptr(ctr, tshift);
+  w_vert = frame_ptr(w_vert, tshift);
+  poly_cnt = frame_ptr(poly_cnt, tshift); poly_gcnt = frame_ptr(poly_gcnt, tshift); poly_excl = frame_ptr(poly_excl, tshift);
+  poly_used = frame_ptr(poly_used, tshift);
+  __shared__ unsigned s_cnt[8][WARPS];
+  __shared__ unsigned s_last;
+  __shared__ unsigned long long s_scan[3][32];
+  __shared__ CutTables s_tab;
+  __shared__ int32_t* s_corners[kMaxFused];   // outputs of the frames of this topology
+  __shared__ int64_t* s_fwt[kMaxFused];
+  __shared__ int64_t s_cap_fwt[kMaxFused];
+  __shared__ int s_nf;
+  load_cut_tables(s_tab);
+  if (threadIdx.x == 32) {
+    int nf = 0;
+    for (unsigned f = 0; f < gridDim.y; ++f) {
+      if (topo.off[f] != tshift) continue;
+      const FwdBlock* b = frame_ptr(blk, fs.off[f]);
+      s_corners[nf] = b->a.tape_corners; s_fwt[nf] = b->a.faces_wt; s_cap_fwt[nf] = b->a.cap_faces_wt;
+      ++nf;
+    }
+    s_nf = nf;
+  }
+  __syncthreads();
+  const int nf = s_nf;
+  const unsigned t1 = tc->work_tri, t2 = tc->work_quad;
+  unsigned long long* tr = trace_begin(tc->trace, tc->trace_frame, K_POLY_FACES);
+  const int64_t npoly = (int64_t)t1 + t2;
+  const int64_t ntiles = (npoly + kPolyThreads - 1) / kPolyThreads;
+  const unsigned ntopo = topo_rows * topo_ctas;
+  const unsigned tile = (blockIdx.y % topo_rows) * topo_ctas + blockIdx.x;
+  // CTAs past the data still take part in the "last CTA out" count (the grid is sized from the capacity)
+  const int64_t i = (int64_t)tile * kPolyThreads + threadIdx.x;
+
+  if ((int64_t)tile < ntiles) {
+    int bucket = -1;
+    if (i < npoly) {
+      const int4 meta = reinterpret_cast<const int4*>(records + i)[1];
+      const int code = meta.x, rank = meta.y;
+      const bool quad = __popc((unsigned)code) == 2;
+      const int n = quad ? 4 : 3;
+      const int64_t p0 = quad ? (3ll * t1 + 4ll * rank) : 3ll * rank;
+      int L[4];
+      float m[4];
+      polygon_corners(static_edges, corners, corner_rank, edge_bits, word_prefix, i, p0, n, L);
+      // the corner array of every frame's tape (poly_cut_kernel and the backward pass read it there)
+      for (int f = 0; f < nf; ++f) {
+        int32_t* __restrict__ dst = s_corners[f];
+        if (static_edges || dst != corners) {
+#pragma unroll
+          for (int k = 0; k < 4; ++k)
+            if (k < n) dst[p0 + k] = L[k];
+        }
+      }
+#pragma unroll
+      for (int k = 0; k < 4; ++k) m[k] = (k < n) ? reinterpret_cast<const float*>(w_vert + L[k])[3] : 0.f;
+      // ---- watertight faces ----
+      const int ntri = quad ? 2 : 1;
+      for (int t = 0; t < ntri; ++t) {
+        const int64_t row = quad ? ((int64_t)t1 + 2ll * rank + t) : (int64_t)rank;
+        int vi[3];
+        triangle_corners(code, t, L, vi);
+        for (int f = 0; f < nf; ++f) {
+          if (row < s_cap_fwt[f]) {
+            int64_t* __restrict__ faces_wt = s_fwt[f];
+            faces_wt[3 * row + 0] = vi[0];
+            faces_wt[3 * row + 1] = vi[1];
+            faces_wt[3 * row + 2] = vi[2];
+          }
+        }
+      }
+      unsigned mcase;
+      int ncut;
+      const float sg = REPLAY ? -1.f : 1.f;  // exact: the pair's interpolated mSDF is the negation (SURVEY A.4)
+      bucket = cut_case(quad, sg * m[0], sg * m[1], sg * m[2], sg * m[3], mcase, ncut);
+      // boundary vertices the cut references (bit k: the one on polygon edge k -> k+1), for the frames' poly_cut CTAs
+      poly_used[i] = (unsigned char)(((quad ? s_tab.uq[mcase] : s_tab.ut[mcase]) >> n) & 0xfu);
+    }
+    // ---- polygons per bucket: per group of 32 polygons (one warp; poly_cut_kernel ranks inside a tile with them) and
+    // per tile of 256 (scanned below by the last CTA).  Lane b keeps the count of bucket b ----
+    unsigned mine = 0u;
+#pragma unroll
+    for (int b = 0; b < 6; ++b) {
+      const unsigned msk = __ballot_sync(0xffffffffu, bucket == b);
+      if (lane == (unsigned)b) mine = __popc(msk);
+    }
+    if (lane < 8u) {   // (entries 6, 7: zero)
+      poly_gcnt[((int64_t)tile * WARPS + warp) * 8 + lane] = mine;
+      s_cnt[lane][warp] = mine;
+    }
+    __syncthreads();
+    if (threadIdx.x < 8) {
+      unsigned run = 0;
+#pragma unroll
+      for (int w = 0; w < WARPS; ++w) run += s_cnt[threadIdx.x][w];
+      poly_cnt[(int64_t)tile * 8 + threadIdx.x] = run;
+    }
+  }
+
+  // ---- last topology CTA out: scan the tile counts, finalise and publish the sizes of every frame of the topology ----
   __threadfence();
   __syncthreads();
   trace_end(tr);
-  if (threadIdx.x == 0) s_last = (atomicAdd(REPLAY ? &ctr->poly_done2 : &ctr->poly_done, 1u) == gridDim.x - 1);
+  if (threadIdx.x == 0) s_last = (atomicAdd(REPLAY ? &tc->poly_done2 : &tc->poly_done, 1u) == ntopo - 1);
   __syncthreads();
   if (!s_last) return;
   __threadfence();
@@ -314,7 +428,11 @@ poly_faces_kernel(const FwdBlock* __restrict__ blk, const d3h_tet_record* __rest
       run[2] += (unsigned long long)c45.x | ((unsigned long long)c45.y << 32);
     }
   }
-  if (threadIdx.x == 0) {
+  // thread f publishes frame f of the launch (if it uses this topology)
+  if (threadIdx.x < gridDim.y && topo.off[threadIdx.x] == tshift) {
+    const int64_t off = fs.off[threadIdx.x];
+    DevCounters* __restrict__ fc = frame_ptr(ctr, off);
+    const FwdBlock* __restrict__ fb = frame_ptr(blk, off);
     unsigned bk[6];
 #pragma unroll
     for (int wd = 0; wd < 3; ++wd) {
@@ -325,23 +443,23 @@ poly_faces_kernel(const FwdBlock* __restrict__ blk, const d3h_tet_record* __rest
     int64_t fa = 0;
     d3h_counts c;
     for (int b = 0; b < 6; ++b) {
-      if (REPLAY) ctr->bucket2[b] = bk[b]; else ctr->bucket[b] = bk[b];
+      if (REPLAY) fc->bucket2[b] = bk[b]; else fc->bucket[b] = bk[b];
       c.bucket_polys[b] = bk[b];
       fa += (int64_t)bk[b] * ncut_of[b];
     }
-    c.n_valid_tets = ctr->n_valid;
-    c.n_tri_tets = ctr->n_tri;
-    c.n_quad_tets = ctr->n_quad;
-    c.n_corners = 3ll * ctr->n_tri + 4ll * ctr->n_quad;
-    c.n_verts = ctr->n_verts;
+    c.n_valid_tets = fc->n_valid;
+    c.n_tri_tets = fc->n_tri;
+    c.n_quad_tets = fc->n_quad;
+    c.n_corners = 3ll * fc->n_tri + 4ll * fc->n_quad;
+    c.n_verts = fc->n_verts;
     c.n_faces_aug = fa;
     c.bad_index = 0;
-    c.overflow = (ctr->n_valid != t1 + t2) ? 1 : 0;  // record buffer overflowed: surface stages skipped
-    const int64_t seq = blk->a.seq;
-    d3h_counts* counts_mapped = blk->counts_mapped;
+    c.overflow = (fc->n_valid != fc->work_tri + fc->work_quad) ? 1 : 0;  // record buffer overflowed: surface stages skipped
+    const int64_t seq = fb->a.seq;
+    d3h_counts* counts_mapped = fb->counts_mapped;
     c.seq = seq;
     c.reserved = 0;
-    *counts_dev = c;
+    *frame_ptr(counts_dev, off) = c;
     if (counts_mapped != nullptr) {  // straight into pinned host memory; `seq` last, after a system-scope fence
       volatile int64_t* dst = reinterpret_cast<volatile int64_t*>(counts_mapped);
       const int64_t* src = reinterpret_cast<const int64_t*>(&c);
@@ -377,89 +495,135 @@ __device__ __forceinline__ float3 vertex_tangent(const float* __restrict__ w_acc
                          __fsub_rn(t.z, __fmul_rn(dp, n.z)));
 }
 
-// Four lanes per polygon (lane k = corner k; the fourth lane of a triangle polygon idles): a 256-thread CTA takes 64
-// polygons = two of poly_faces_kernel's 32-polygon groups.  Every lane evaluates ONE vertex frame and ONE boundary
-// vertex and writes at most one cut triangle; the values of the neighbouring corner travel by warp shuffles.  (v1 gave
-// a whole polygon to one thread: four vertex frames in sequence on 226 CTAs, 14 us for 58 k polygons.)
-constexpr int kCutPolysPerCta = kPolyThreads / 4;
-
-// cut tables as shared-memory words (the case code differs from lane to lane: __constant__ would serialise)
-struct CutTables {
-  unsigned long long quad[16];   // 12 locals x 4 bits
-  unsigned tri[8];               //  6 locals x 4 bits
-  unsigned char nq[16], nt[8];   // number of cut triangles
-  unsigned char uq[16], ut[8];   // locals referenced by the cut triangles (bit mask)
-};
-
-__device__ __forceinline__ void load_cut_tables(CutTables& T) {
-  const unsigned t = threadIdx.x;
-  if (t < 16u) {
-    unsigned long long w = 0ull;
-    unsigned used = 0u;
-    const int n = c_num_cut_quad[t];
-    for (int e = 0; e < 12; ++e) {
-      const int loc = c_cut_quad[t][e];
-      w |= (unsigned long long)(loc & 0xf) << (4 * e);
-      if (e < 3 * n) used |= 1u << loc;
-    }
-    T.quad[t] = w; T.nq[t] = (unsigned char)n; T.uq[t] = (unsigned char)used;
-  } else if (t < 24u) {
-    const unsigned c = t - 16u;
-    unsigned w = 0u, used = 0u;
-    const int n = c_num_cut_tri[c];
-    for (int e = 0; e < 6; ++e) {
-      const int loc = c_cut_tri[c][e];
-      w |= (unsigned)(loc & 0xf) << (4 * e);
-      if (e < 3 * n) used |= 1u << loc;
-    }
-    T.tri[c] = w; T.nt[c] = (unsigned char)n; T.ut[c] = (unsigned char)used;
-  }
-}
-
 template <bool REPLAY>
 __global__ void __launch_bounds__(kPolyThreads, D3H_CUT_MINB)
 poly_cut_kernel(const FwdBlock* __restrict__ blk, const d3h_tet_record* __restrict__ records,
                 const DevCounters* __restrict__ ctr, const float4* __restrict__ w_vert,
                 const float* __restrict__ w_acc, const int32_t* __restrict__ owner,
-                const unsigned* __restrict__ poly_gcnt, const unsigned* __restrict__ poly_excl, const __grid_constant__ FrameSet fs,
-                const __grid_constant__ FrameSet topo) {
+                const unsigned* __restrict__ poly_gcnt, const unsigned* __restrict__ poly_excl,
+                const unsigned char* __restrict__ poly_used, unsigned topo_ctas, unsigned topo_rows,
+                const __grid_constant__ FrameSet fs, const __grid_constant__ FrameSet topo) {
   pdl_enter();
-  {
-    const int64_t shift = fs.off[blockIdx.y];
-    records = frame_ptr(records, topo.off[blockIdx.y]);   // (shared topology: the first frame's records)
-    blk = frame_ptr(blk, shift); ctr = frame_ptr(ctr, shift);
-    w_vert = frame_ptr(w_vert, shift); w_acc = frame_ptr(w_acc, shift); owner = frame_ptr(owner, shift);
-    poly_gcnt = frame_ptr(poly_gcnt, shift); poly_excl = frame_ptr(poly_excl, shift);
-  }
   constexpr int WARPS = kPolyThreads / 32;
   constexpr unsigned FULL = 0xffffffffu;
-  const int32_t* __restrict__ corners = blk->a.tape_corners;
-  float* __restrict__ verts_aug = blk->a.verts_aug;
-  float* __restrict__ v_tng_aug = blk->a.v_tng_aug;
-  float* __restrict__ msdf_aug = blk->a.msdf_aug;
-  float* __restrict__ v_tng_wt = blk->a.v_tng_wt;
-  int64_t* __restrict__ faces_aug = blk->a.faces_aug;
-  const int64_t cap_verts_aug = blk->a.cap_verts_aug, cap_verts = blk->a.cap_verts, cap_faces_aug = blk->a.cap_faces_aug;
+  const int64_t shift = fs.off[blockIdx.y], tshift = topo.off[blockIdx.y];
+  records = frame_ptr(records, tshift);   // (shared topology: the first frame's records and corner ids)
+  const int32_t* __restrict__ corners = frame_ptr(blk, tshift)->a.tape_corners;
+  const unsigned lane = lane_id(), warp = threadIdx.x >> 5;
+  const unsigned k = lane & 3u, lane0 = lane & ~3u;                 // corner of this lane, first lane of its polygon
+
+  if (blockIdx.x >= topo_ctas) {
+    // ---- the frame's own CTAs: vertex frames, tangent rows and the boundary vertices' positions and tangents ----
+    blk = frame_ptr(blk, shift); ctr = frame_ptr(ctr, shift);
+    w_vert = frame_ptr(w_vert, shift); w_acc = frame_ptr(w_acc, shift); owner = frame_ptr(owner, shift);
+    poly_used = frame_ptr(poly_used, tshift);
+    float* __restrict__ verts_aug = blk->a.verts_aug;
+    float* __restrict__ v_tng_aug = blk->a.v_tng_aug;
+    float* __restrict__ v_tng_wt = blk->a.v_tng_wt;
+    const int64_t cap_verts_aug = blk->a.cap_verts_aug, cap_verts = blk->a.cap_verts;
+    const bool static_edges = blk->a.edge_off != nullptr;
+    const unsigned t1 = ctr->work_tri, t2 = ctr->work_quad;
+    unsigned long long* tr = trace_begin(ctr->trace, ctr->trace_frame, K_POLY_CUT);
+    const int64_t npoly = (int64_t)t1 + t2;
+    const unsigned tile = blockIdx.x - topo_ctas;
+    if ((int64_t)tile * kCutPolysPerCta >= npoly) return;
+    const int64_t nv = ctr->n_verts;
+    const int64_t i = (int64_t)tile * kCutPolysPerCta + warp * 8 + (lane >> 2);
+    bool corner = false;
+    int n = 3;
+    int64_t p0 = 0;
+    unsigned used = 0u;
+    float4 P = make_float4(0.f, 0.f, 0.f, 0.f);
+    float3 T = make_float3(0.f, 0.f, 0.f);
+    if (i < npoly) {
+      const int4 meta = reinterpret_cast<const int4*>(records + i)[1];
+      const int code = meta.x, rank = meta.y;
+      const bool quad = __popc((unsigned)code) == 2;
+      n = quad ? 4 : 3;
+      p0 = quad ? (3ll * t1 + 4ll * rank) : 3ll * rank;
+      corner = (int)k < n;
+      if (corner) {
+        used = (poly_used[i] >> k) & 1u;
+        const int L = corners[p0 + k];
+        P = w_vert[L];
+        if (REPLAY) P.w = -P.w;  // the pair's interpolated mSDF: exact negation
+        T = vertex_tangent(w_acc, L);
+        // the corner that opened the vertex's run in the sorted key array writes the vertex's own tangent rows
+        // (static edge table paths: no owner is known, every corner writes the same value)
+        if (static_edges || owner[L] == (int32_t)(p0 + k)) {
+          const int64_t v = L;
+          if (v < cap_verts) {
+            store_same_value(v_tng_wt + 3 * v, T.x);
+            store_same_value(v_tng_wt + 3 * v + 1, T.y);
+            store_same_value(v_tng_wt + 3 * v + 2, T.z);
+          }
+          if (v < cap_verts_aug) {
+            store_same_value(v_tng_aug + 3 * v, T.x);
+            store_same_value(v_tng_aug + 3 * v + 1, T.y);
+            store_same_value(v_tng_aug + 3 * v + 2, T.z);
+          }
+        }
+      }
+    }
+    // ---- boundary vertex on polygon edge k -> k+1: this lane's corner and the next one's ----
+    const unsigned kn = ((int)k + 1 == n) ? 0u : k + 1u;
+    const unsigned src = lane0 + (corner ? kn : k);
+    float4 Pj;
+    float3 Tj;
+    Pj.x = __shfl_sync(FULL, P.x, src); Pj.y = __shfl_sync(FULL, P.y, src);
+    Pj.z = __shfl_sync(FULL, P.z, src); Pj.w = __shfl_sync(FULL, P.w, src);
+    Tj.x = __shfl_sync(FULL, T.x, src); Tj.y = __shfl_sync(FULL, T.y, src); Tj.z = __shfl_sync(FULL, T.z, src);
+    if (corner) {
+      float u0, u1, D;
+      boundary_weights(P.w, Pj.w, u0, u1, D);
+      const int64_t row = nv + p0 + k;
+      if (row < cap_verts_aug) {
+        if (used) {   // (the topology CTAs zero the rows of the others)
+          verts_aug[3 * row + 0] = lerp2(P.x, u0, Pj.x, u1);
+          verts_aug[3 * row + 1] = lerp2(P.y, u0, Pj.y, u1);
+          verts_aug[3 * row + 2] = lerp2(P.z, u0, Pj.z, u1);
+        }
+        v_tng_aug[3 * row + 0] = lerp2(T.x, u0, Tj.x, u1);
+        v_tng_aug[3 * row + 1] = lerp2(T.y, u0, Tj.y, u1);
+        v_tng_aug[3 * row + 2] = lerp2(T.z, u0, Tj.z, u1);
+      }
+    }
+    trace_end(tr);
+    return;
+  }
+
+  // ---- topology CTAs: cut case, rank of the polygon in its bucket, and for every frame of the topology its faces_aug
+  // rows, the boundary mSDF and the zero rows of the boundary vertices no cut triangle references ----
+  ctr = frame_ptr(ctr, tshift); w_vert = frame_ptr(w_vert, tshift);
+  poly_gcnt = frame_ptr(poly_gcnt, tshift); poly_excl = frame_ptr(poly_excl, tshift);
   __shared__ unsigned s_cnt[6][WARPS];
   __shared__ CutTables s_tab;
-  const bool static_edges = blk->a.edge_off != nullptr;
+  __shared__ CutOut s_out[kMaxFused];
+  __shared__ int s_nf;
   const unsigned t1 = ctr->work_tri, t2 = ctr->work_quad;
   unsigned long long* tr = trace_begin(ctr->trace, ctr->trace_frame, K_POLY_CUT);
   const int64_t npoly = (int64_t)t1 + t2;
-  const unsigned tile = blockIdx.x;
+  const unsigned tile = (blockIdx.y % topo_rows) * topo_ctas + blockIdx.x;
   if ((int64_t)tile * kCutPolysPerCta >= npoly) return;
   load_cut_tables(s_tab);
+  if (threadIdx.x == 32) {
+    int nf = 0;
+    for (unsigned f = 0; f < gridDim.y; ++f) {
+      if (topo.off[f] != tshift) continue;
+      const FwdBlock* b = frame_ptr(blk, fs.off[f]);
+      s_out[nf] = CutOut{b->a.faces_aug, b->a.verts_aug, b->a.msdf_aug, b->a.cap_faces_aug, b->a.cap_verts_aug};
+      ++nf;
+    }
+    s_nf = nf;
+  }
   const int64_t nv = ctr->n_verts;
-  const unsigned lane = lane_id(), warp = threadIdx.x >> 5;
-  const unsigned k = lane & 3u, lane0 = lane & ~3u;                 // corner of this lane, first lane of its polygon
   const int64_t i = (int64_t)tile * kCutPolysPerCta + warp * 8 + (lane >> 2);
   const bool live = i < npoly;
 
   bool quad = false, corner = false;
   int n = 3, L = 0;
   int64_t p0 = 0;
-  float4 P = make_float4(0.f, 0.f, 0.f, 0.f);
-  float3 T = make_float3(0.f, 0.f, 0.f);
+  float m = 0.f;
   if (live) {
     const int4 meta = reinterpret_cast<const int4*>(records + i)[1];
     const int code = meta.x, rank = meta.y;
@@ -469,29 +633,13 @@ poly_cut_kernel(const FwdBlock* __restrict__ blk, const d3h_tet_record* __restri
     corner = (int)k < n;
     if (corner) {
       L = corners[p0 + k];
-      P = w_vert[L];
-      if (REPLAY) P.w = -P.w;  // the pair's interpolated mSDF: exact negation
-      T = vertex_tangent(w_acc, L);
-      // the corner that opened the vertex's run in the sorted key array writes the vertex's own tangent rows
-      // (static edge table paths: no owner is known, every corner writes the same value)
-      if (static_edges || owner[L] == (int32_t)(p0 + k)) {
-        const int64_t v = L;
-        if (v < cap_verts) {
-          store_same_value(v_tng_wt + 3 * v, T.x);
-          store_same_value(v_tng_wt + 3 * v + 1, T.y);
-          store_same_value(v_tng_wt + 3 * v + 2, T.z);
-        }
-        if (v < cap_verts_aug) {
-          store_same_value(v_tng_aug + 3 * v, T.x);
-          store_same_value(v_tng_aug + 3 * v + 1, T.y);
-          store_same_value(v_tng_aug + 3 * v + 2, T.z);
-        }
-      }
+      m = reinterpret_cast<const float*>(w_vert + L)[3];
+      if (REPLAY) m = -m;  // the pair's interpolated mSDF: exact negation
     }
   }
-  __syncthreads();   // the tables
+  __syncthreads();   // the tables and the outputs
   // ---- mSDF cut case from the four corner signs (gshell_tets.py:338-339, 401-404) ----
-  const unsigned mo = (__ballot_sync(FULL, corner && P.w > 0.f) >> lane0) & 0xfu;   // bit c = corner c
+  const unsigned mo = (__ballot_sync(FULL, corner && m > 0.f) >> lane0) & 0xfu;   // bit c = corner c
   unsigned mcase;
   int ncut = 0, bucket = -1;
   unsigned used_mask = 0u;
@@ -509,9 +657,9 @@ poly_cut_kernel(const FwdBlock* __restrict__ blk, const d3h_tet_record* __restri
   unsigned my_ballot = 0;
 #pragma unroll
   for (int b = 0; b < 6; ++b) {
-    const unsigned m = __ballot_sync(FULL, bucket == b && k == 0u);
-    if (bucket == b) my_ballot = m;
-    if (lane == 0) s_cnt[b][warp] = __popc(m);
+    const unsigned msk = __ballot_sync(FULL, bucket == b && k == 0u);
+    if (bucket == b) my_ballot = msk;
+    if (lane == 0) s_cnt[b][warp] = __popc(msk);
   }
   __syncthreads();
   int64_t row0 = 0;
@@ -529,27 +677,26 @@ poly_cut_kernel(const FwdBlock* __restrict__ blk, const d3h_tet_record* __restri
     for (unsigned w = warp & ~3u; w < warp; ++w) before += s_cnt[bucket][w];
     row0 = fbase + ((int64_t)before + __popc(my_ballot & ((1u << lane0) - 1u))) * ncut;   // polygons before this one
   }
-  // ---- boundary vertex on polygon edge k -> k+1: this lane's corner and the next one's ----
+  const int nf = s_nf;
+  // ---- boundary vertex on polygon edge k -> k+1: its mSDF, and a zero row where no cut triangle references it ----
   const unsigned kn = ((int)k + 1 == n) ? 0u : k + 1u;
-  const unsigned src = lane0 + (corner ? kn : k);
-  float4 Pj;
-  float3 Tj;
-  Pj.x = __shfl_sync(FULL, P.x, src); Pj.y = __shfl_sync(FULL, P.y, src);
-  Pj.z = __shfl_sync(FULL, P.z, src); Pj.w = __shfl_sync(FULL, P.w, src);
-  Tj.x = __shfl_sync(FULL, T.x, src); Tj.y = __shfl_sync(FULL, T.y, src); Tj.z = __shfl_sync(FULL, T.z, src);
+  const float mj = __shfl_sync(FULL, m, lane0 + (corner ? kn : k));
   if (corner) {
     float u0, u1, D;
-    boundary_weights(P.w, Pj.w, u0, u1, D);
+    boundary_weights(m, mj, u0, u1, D);
     const int64_t row = nv + p0 + k;
-    if (row < cap_verts_aug) {
-      const bool used = (used_mask >> (n + k)) & 1u;
-      verts_aug[3 * row + 0] = used ? lerp2(P.x, u0, Pj.x, u1) : 0.f;
-      verts_aug[3 * row + 1] = used ? lerp2(P.y, u0, Pj.y, u1) : 0.f;
-      verts_aug[3 * row + 2] = used ? lerp2(P.z, u0, Pj.z, u1) : 0.f;
-      v_tng_aug[3 * row + 0] = lerp2(T.x, u0, Tj.x, u1);
-      v_tng_aug[3 * row + 1] = lerp2(T.y, u0, Tj.y, u1);
-      v_tng_aug[3 * row + 2] = lerp2(T.z, u0, Tj.z, u1);
-      msdf_aug[row] = lerp2(P.w, u0, Pj.w, u1);
+    const bool used = (used_mask >> (n + k)) & 1u;
+    const float mb = lerp2(m, u0, mj, u1);
+    for (int f = 0; f < nf; ++f) {
+      const CutOut o = s_out[f];
+      if (row < o.cap_verts_aug) {
+        if (!used) {
+          o.verts_aug[3 * row + 0] = 0.f;
+          o.verts_aug[3 * row + 1] = 0.f;
+          o.verts_aug[3 * row + 2] = 0.f;
+        }
+        o.msdf_aug[row] = mb;
+      }
     }
   }
   // ---- cut triangles: lane k writes triangle k of its polygon ----
@@ -562,7 +709,8 @@ poly_cut_kernel(const FwdBlock* __restrict__ blk, const d3h_tet_record* __restri
     if (tri_here) {
       const int64_t g = is_corner ? (int64_t)Lv : nv + p0 + (loc - n);
       const int64_t frow = row0 + k;
-      if (frow < cap_faces_aug) faces_aug[3 * frow + c] = g;
+      for (int f = 0; f < nf; ++f)
+        if (frow < s_out[f].cap_faces_aug) s_out[f].faces_aug[3 * frow + c] = g;
     }
   }
   trace_end(tr);
@@ -611,6 +759,14 @@ static unsigned cut_blocks(const Workspace& ws) {
   return (unsigned)(n > 0 ? n : 1);
 }
 
+// Rows of the launch that split the tiles of one topology (all of them when the frames share it, see poly_faces_kernel),
+// and the topology CTAs each of them takes out of `tiles`.
+static unsigned topo_rows() {
+  const BatchCtx& ctx = batch_ctx();
+  return ctx.topo_frames == 1 ? (unsigned)ctx.frames : 1u;
+}
+static unsigned topo_ctas(unsigned tiles, unsigned rows) { return (tiles + rows - 1) / rows; }
+
 void launch_surface(const d3h_forward_args& a, const Workspace& ws, const d3h_tet_record* records,
                     cudaStream_t stream) {
   const UvParams uvp = uv_params(a.n_tets);
@@ -619,16 +775,19 @@ void launch_surface(const d3h_forward_args& a, const Workspace& ws, const d3h_te
     launch_k(publish_counts_kernel, 1u, 1u, stream, kLaunchLatency, ws.blk, ws.ctr, ws.counts);
     return;
   }
-  const unsigned nblk = (unsigned)(ws.ntiles_poly > 0 ? ws.ntiles_poly : 1);
+  const unsigned rows = topo_rows();
+  const unsigned nblk = (unsigned)(ws.ntiles_poly > 0 ? ws.ntiles_poly : 1), ncut = cut_blocks(ws);
+  const unsigned tfaces = topo_ctas(nblk, rows), tcut = topo_ctas(ncut, rows);
   {
     ProfScope ps(K_POLY_FACES, stream);
-    launch_k_dep(poly_faces_kernel<false>, nblk, (unsigned)kPolyThreads, stream, kLaunchLatency, ws.blk, records, ws.ctr,
-                 ws.vert, ws.acc, ws.poly_cnt, ws.poly_gcnt, ws.poly_excl, uvp, ws.counts, ws.corner_rank, ws.edge_bits,
-                 ws.word_prefix, batch_ctx().fs, batch_ctx().topo);
+    launch_k_dep(poly_faces_kernel<false>, tfaces + nblk, (unsigned)kPolyThreads, stream, kLaunchLatency, ws.blk, records,
+                 ws.ctr, ws.vert, ws.acc, ws.poly_cnt, ws.poly_gcnt, ws.poly_excl, ws.poly_used, uvp, ws.counts,
+                 ws.corner_rank, ws.edge_bits, ws.word_prefix, tfaces, rows, batch_ctx().fs, batch_ctx().topo);
   }
   ProfScope ps(K_POLY_CUT, stream);
-  launch_k_dep(poly_cut_kernel<false>, cut_blocks(ws), (unsigned)kPolyThreads, stream, kLaunchLatency, ws.blk, records, ws.ctr,
-           ws.vert, ws.acc, ws.owner, ws.poly_gcnt, ws.poly_excl, batch_ctx().fs, batch_ctx().topo);
+  launch_k_dep(poly_cut_kernel<false>, tcut + ncut, (unsigned)kPolyThreads, stream, kLaunchLatency, ws.blk, records, ws.ctr,
+               ws.vert, ws.acc, ws.owner, ws.poly_gcnt, ws.poly_excl, ws.poly_used, tcut, rows, batch_ctx().fs,
+               batch_ctx().topo);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -865,12 +1024,13 @@ void launch_pair_replay(const d3h_forward_args& a, const Workspace& ws, const d3
     return;
   }
   const UvParams uvp = uv_params(a.n_tets);
-  const unsigned nblk = (unsigned)(ws.ntiles_poly > 0 ? ws.ntiles_poly : 1);
+  // one frame: topology CTAs only in poly_faces_kernel (no normals / tangents to splat), both kinds in poly_cut_kernel
+  const unsigned nblk = (unsigned)(ws.ntiles_poly > 0 ? ws.ntiles_poly : 1), ncut = cut_blocks(ws);
   launch_k(poly_faces_kernel<true>, nblk, (unsigned)kPolyThreads, stream, kLaunchLatency, ws.blk2, records, ws.ctr, ws.vert,
-           ws.acc, ws.poly_cnt, ws.poly_gcnt, ws.poly_excl, uvp, ws.counts2, ws.corner_rank, ws.edge_bits, ws.word_prefix,
-           FrameSet{}, FrameSet{});
-  launch_k(poly_cut_kernel<true>, cut_blocks(ws), (unsigned)kPolyThreads, stream, kLaunchLatency, ws.blk2, records, ws.ctr,
-           ws.vert, ws.acc, ws.owner, ws.poly_gcnt, ws.poly_excl, FrameSet{}, FrameSet{});
+           ws.acc, ws.poly_cnt, ws.poly_gcnt, ws.poly_excl, ws.poly_used, uvp, ws.counts2, ws.corner_rank, ws.edge_bits,
+           ws.word_prefix, nblk, 1u, FrameSet{}, FrameSet{});
+  launch_k(poly_cut_kernel<true>, 2 * ncut, (unsigned)kPolyThreads, stream, kLaunchLatency, ws.blk2, records, ws.ctr,
+           ws.vert, ws.acc, ws.owner, ws.poly_gcnt, ws.poly_excl, ws.poly_used, ncut, 1u, FrameSet{}, FrameSet{});
 }
 
 }  // namespace d3h
