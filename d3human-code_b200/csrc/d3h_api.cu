@@ -846,8 +846,9 @@ static int check_backward_args(const d3h_backward_args* a, const char* who) {
 }
 
 // Adjoints of a batch.  Gradient buffers may be shared between frames (sdf / msdf of a batch of video frames are the
-// same tensors): every frame accumulates with atomics, so a shared buffer ends up with the sum over the frames.  A
-// shared buffer must be zero on entry (grads_prezeroed = 1 on every frame that uses it).
+// same tensors): every frame accumulates with atomics, so a shared buffer ends up with the sum over the frames.  With
+// grads_prezeroed = 0 the call zeroes such a buffer once, before any frame accumulates into it; with grads_prezeroed = 1
+// on every frame that uses it, it must be zero on entry.
 extern "C" int d3h_extract_backward_batch(const d3h_backward_args* args, int64_t n_frames, int32_t lanes,
                                           d3h_stream_t s) {
   if (!args || n_frames < 0 || lanes < 1) { set_error("d3h_extract_backward_batch: null args / bad sizes"); return D3H_E_BADARG; }

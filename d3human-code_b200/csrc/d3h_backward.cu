@@ -1,7 +1,10 @@
 // Backward of the float pipeline (the reference relies on autograd through gshell_tets.py:291-303, 342-397, 427).
 //
-//   zero_kernel    : dense (N,3)+(N)+(N) gradients, one launch, 16-byte stores.  Normally enqueued by the FORWARD call
-//                    (d3h_forward_args.zero_g_*) behind the size publication, where it overlaps the host's wake-up.
+//   zero_rows_kernel : dense (N,3)+(N)+(N) gradients of every frame of a backward call whose buffers were not pre-zeroed,
+//                    ONE launch (grid.y = frame) ahead of the adjoints, 16-byte stores.  A training step's host work
+//                    between two extractions leaves the GPU idle around the backward call, while the forward rounds are
+//                    its critical path, so the fill runs here.  The forward call can still do it instead
+//                    (d3h_forward_args.zero_g_*, zero_block_kernel; single calls and the tet-sharded path do).
 //   adjoint_kernel : one thread per watertight vertex v (= crossing edge (a,b), sorted by a).  The forward sort left, for
 //                    every vertex, the list of polygon corners that reference it (tape_runs / tape_slots), so the
 //                    boundary-vertex adjoints are GATHERED: for each corner the thread evaluates the two polygon edges
@@ -21,6 +24,7 @@
 //
 // Gradient formulas: SURVEY.md appendix A.5 (verified against the reference's autograd in tests/).
 #include <cstdlib>
+#include <unordered_set>
 
 #include "d3h_internal.cuh"
 
@@ -41,12 +45,25 @@ __device__ __forceinline__ void zero_span(float* __restrict__ p, int64_t len, in
   if (tid < len - t0) p[t0 + tid] = 0.f;
 }
 
-__global__ void __launch_bounds__(256) zero_kernel(float* p0, int64_t n0, float* p1, int64_t n1, float* p2, int64_t n2) {
+// One row of the backward zero-fill: the gradient buffers one frame of the call zeroes (nullptr: none, or another row
+// has it) and their grid size.
+struct ZeroRow {
+  float *g_pos, *g_sdf, *g_msdf;
+  int64_t n;
+};
+constexpr int kZeroRows = 128;     // rows per launch (4 KB of kernel parameters): the largest batch extract.py makes
+struct ZeroBatch {
+  ZeroRow r[kZeroRows];
+};
+
+// grid.y = row
+__global__ void __launch_bounds__(256) zero_rows_kernel(const __grid_constant__ ZeroBatch zb) {
+  const ZeroRow& r = zb.r[blockIdx.y];
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   const int64_t tid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  zero_span(p0, n0, tid, stride);
-  zero_span(p1, n1, tid, stride);
-  zero_span(p2, n2, tid, stride);
+  zero_span(r.g_pos, 3 * r.n, tid, stride);
+  zero_span(r.g_sdf, r.n, tid, stride);
+  zero_span(r.g_msdf, r.n, tid, stride);
 }
 
 // Forward-side variant: the three pointers come from the argument block (they change from call to call, the launch
@@ -69,7 +86,8 @@ void launch_zero_grads_from_block(const d3h_forward_args& a, const Workspace& ws
   // A fused batch runs the fill on a side stream next to the latency-bound kernels of the main chain.  A small launch (a
   // few CTAs per SM that keep HBM busy without taking the CTA slots of those kernels) was measured and is SLOWER: 1.51 /
   // 1.34-1.40 / 1.27 ms per step with 148 / 296 / 592 CTAs against 1.22 ms with 1184 or the full grid (r02at).
-  // D3H_ZERO_CTAS = CTAs of the whole launch (A/B); default: no cap.
+  // D3H_ZERO_CTAS = CTAs of the whole launch (A/B of this forward placement, which batches take with
+  // D3H_ZERO_IN_FORWARD=1; extract.py); default: no cap.
   const int frames = batch_ctx().frames;
   if (frames > 1) {
     static int total = -1;
@@ -86,13 +104,51 @@ void launch_zero_grads_from_block(const d3h_forward_args& a, const Workspace& ws
   launch_k(zero_block_kernel, (unsigned)blocks, 256u, stream, kLaunchLatency, ws.blk, a.n_grid, batch_ctx().fs);
 }
 
-void launch_zero_grads(float* g_pos, float* g_sdf, float* g_msdf, int64_t n, cudaStream_t stream) {
-  int64_t blocks = (5 * n / 16 + 255) / 256;
+static void launch_zero_rows(const ZeroBatch& zb, int m, int64_t max_n, cudaStream_t stream) {
+  int64_t blocks = (5 * max_n / 16 + 255) / 256;
   if (blocks < 1) blocks = 1;
   if (blocks > 148 * 8) blocks = 148 * 8;
   ProfScope ps(K_ZERO, stream);
-  launch_k(zero_kernel, (unsigned)blocks, 256u, stream, kLaunchStream, g_pos, g_pos ? 3 * n : (int64_t)0, g_sdf,
-           g_sdf ? n : (int64_t)0, g_msdf, g_msdf ? n : (int64_t)0);
+  cudaLaunchConfig_t cfg;
+  memset(&cfg, 0, sizeof(cfg));
+  cfg.gridDim = dim3((unsigned)blocks, (unsigned)m, 1);
+  cfg.blockDim = dim3(256, 1, 1);
+  cfg.stream = stream;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributePriority;
+  at[0].val.priority = launch_priority(kLaunchStream);   // HBM-bound: the latency-bound kernels of other streams go first
+  cfg.attrs = at;
+  cfg.numAttrs = 1;
+  cudaLaunchKernelEx(&cfg, zero_rows_kernel, zb);
+}
+
+// Zero-fill of the gradient buffers of every frame with grads_prezeroed = 0, in ONE launch per kZeroRows frames ahead of
+// the adjoints.  A buffer several frames share (sdf / msdf of a batch of video frames) is zeroed once, by its first frame.
+static void launch_zero_grads(const d3h_backward_args* a, int64_t n, cudaStream_t stream) {
+  ZeroBatch zb;
+  memset(&zb, 0, sizeof(zb));
+  int m = 0;
+  int64_t max_n = 0;
+  std::unordered_set<const float*> seen;
+  auto first = [&](float* p) { return (p != nullptr && seen.insert(p).second) ? p : nullptr; };
+  for (int64_t i = 0; i < n; ++i) {
+    if (a[i].grads_prezeroed) continue;
+    ZeroRow r;
+    r.g_pos = first(a[i].g_pos);
+    r.g_sdf = first(a[i].g_sdf);
+    r.g_msdf = first(a[i].g_msdf);
+    r.n = a[i].n_grid;
+    if (!r.g_pos && !r.g_sdf && !r.g_msdf) continue;
+    zb.r[m++] = r;
+    if (r.n > max_n) max_n = r.n;
+    if (m == kZeroRows) {
+      launch_zero_rows(zb, m, max_n, stream);
+      memset(&zb, 0, sizeof(zb));
+      m = 0;
+      max_n = 0;
+    }
+  }
+  if (m > 0) launch_zero_rows(zb, m, max_n, stream);
 }
 
 // segmented (by key) inclusive suffix-sum inside a warp; lanes with equal key must be contiguous.
@@ -353,18 +409,23 @@ static AdjFrame adj_frame(const d3h_backward_args& a) {
   return f;
 }
 
-// Adjoints of n frames: zero-fills first where the caller did not pre-zero, then ONE adjoint launch per kAdjBatch frames
-// (grid.y = frame).
+static bool has_upstream(const d3h_backward_args& a) {
+  return a.g_verts_aug || a.g_msdf_aug || a.g_msdf_boundary || a.g_verts_wt || a.g_msdf_wt || a.g_verts_tng ||
+         a.g_mvert_tng;
+}
+
+// Adjoints of n frames: the zero-fill first (frames that were not pre-zeroed), then ONE adjoint launch per kAdjBatch
+// consecutive frames (grid.y = frame).  A frame with no surface or no upstream gradient gets no row of the launch, so a
+// call of blocks without upstream gradients is a zero-fill alone (extract.py zeroes a batch's buffers that way).
 void launch_backward_batch(const d3h_backward_args* a, int64_t n, cudaStream_t stream) {
-  for (int64_t i = 0; i < n; ++i)
-    if (!a[i].grads_prezeroed) launch_zero_grads(a[i].g_pos, a[i].g_sdf, a[i].g_msdf, a[i].n_grid, stream);
+  launch_zero_grads(a, n, stream);
   for (int64_t i0 = 0; i0 < n; i0 += kAdjBatch) {
     AdjBatch batch;
     memset(&batch, 0, sizeof(batch));
     int m = 0;
     int64_t max_nv = 0, max_poly = 0;
     for (int64_t i = i0; i < n && i < i0 + kAdjBatch; ++i) {
-      if (a[i].n_verts <= 0) continue;
+      if (a[i].n_verts <= 0 || !has_upstream(a[i])) continue;
       batch.f[m++] = adj_frame(a[i]);
       if (a[i].n_verts > max_nv) max_nv = a[i].n_verts;
       const bool scatter = a[i].tape_slots == nullptr && a[i].vacc != nullptr;

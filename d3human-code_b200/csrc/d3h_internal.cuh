@@ -143,7 +143,6 @@ void launch_pair_replay(const d3h_forward_args& a, const Workspace& ws, const d3
                         cudaStream_t stream);
 void launch_rank_records(const d3h_forward_args& a, const Workspace& ws, d3h_tet_record* records, int64_t n_records,
                          cudaStream_t stream);
-void launch_zero_grads(float* g_pos, float* g_sdf, float* g_msdf, int64_t n_grid, cudaStream_t stream);
 void launch_zero_grads_from_block(const d3h_forward_args& a, const Workspace& ws, cudaStream_t stream);
 void launch_backward(const d3h_backward_args& a, cudaStream_t stream);
 void launch_backward_batch(const d3h_backward_args* a, int64_t n, cudaStream_t stream);

@@ -469,7 +469,8 @@ def _r4(n: int) -> int:
 _WAIT_TIMEOUT_US = 60_000_000
 
 #: kernels one forward extraction enqueues: prepare, classify, compact, bucket_scan, partition, group_sort, vertex_emit,
-#: poly_faces, poly_cut (+ zero_block_kernel when the gradient buffers are pre-zeroed); backward: adjoint_kernel
+#: poly_faces, poly_cut (+ zero_block_kernel with D3H_ZERO_IN_FORWARD=1); backward: the zero-fill (a batch, unless the
+#: forward call did it) + adjoint_kernel
 LAUNCHES_FORWARD = 9
 #: static edge table path: prepare, classify, compact, edge_emit, poly_faces, poly_cut; backward: adjoint_poly + adjoint
 LAUNCHES_FORWARD_STATIC = 6
@@ -569,7 +570,8 @@ class _Layout:
 
 class _Pending:
     """A batch whose forward kernels have been enqueued but whose sizes have not been read yet."""
-    __slots__ = ("inputs", "plan", "lay", "fslab", "islab", "tape", "seq0", "slot0", "bmat", "launches", "dev", "B")
+    __slots__ = ("inputs", "plan", "lay", "fslab", "islab", "tape", "seq0", "slot0", "bmat", "zero_bwd", "launches", "dev",
+                 "B")
 
 
 _unjoined: Dict[Any, bool] = {}   # device index -> a batch was launched without joining the lanes yet
@@ -584,7 +586,9 @@ def _launch_frames(ptrs, negate, dev, n_grid: int, tets_i32: torch.Tensor, water
 
     ptrs   : (B,3) int64 array (or nested list): per frame the device pointers of pos / sdf / msdf -- contiguous fp32
              data, sdf / msdf 16-byte aligned (the caller keeps the tensors alive); negate: per-frame msdf_negate flags
-    zero   : (B,3) pointers (0 = none) of dense gradient buffers the call zero-fills for the coming backward pass
+    zero   : (B,3) pointers (0 = none) of the dense gradient buffers to zero-fill for the coming backward pass, each
+             buffer under one frame.  With D3H_ZERO_IN_FORWARD=1 this call fills them, otherwise the backward pass
+             does (_zero_backward)
     grad_ptrs : (B,3) pointers of the gradient buffers (pos, sdf, msdf); when given, the d3h_backward_args of the batch
              are prefilled here (everything but the upstream gradients and the sizes is known already)
     launcher : replaces the library call (tet-range sharding, sharding.py): launcher(A, plan, stream) enqueues the work
@@ -655,7 +659,7 @@ def _launch_frames(ptrs, negate, dev, n_grid: int, tets_i32: torch.Tensor, water
             if static is not None:
                 A[:, c["vacc"]] = lay.vacc_off + bases[0]
             launches = B * forward_launches(static, ct)
-            if zero is not None:
+            if zero is not None and _zero_in_forward():
                 A[:, c["zero_g_pos"]:c["zero_g_msdf"] + 1] = zero
                 launches += int(np.count_nonzero(np.asarray(zero).any(axis=1)))
             else:
@@ -670,7 +674,7 @@ def _launch_frames(ptrs, negate, dev, n_grid: int, tets_i32: torch.Tensor, water
                                  ("pair_msdf_wt", "msdf_wt"), ("pair_faces_wt", "faces_wt"), ("pair_vacc", "vacc"),
                                  ("pair_counts_host", "counts_host"), ("pair_seq", "seq")):
                     A[0, c[dst]] = A[1, c[src]]
-                if zero is not None:   # one call: every zero-fill duty moves to frame 0 (a buffer has one duty holder)
+                if zero is not None and _zero_in_forward():   # one call: every zero-fill duty moves to frame 0
                     z = np.asarray(zero, dtype=np.int64)
                     A[0, c["zero_g_pos"]:c["zero_g_msdf"] + 1] = z[0] | z[1]
                     A[1, c["zero_g_pos"]:c["zero_g_msdf"] + 1] = 0
@@ -718,6 +722,7 @@ def _launch_frames(ptrs, negate, dev, n_grid: int, tets_i32: torch.Tensor, water
                 bmat[:, b["vacc"]] = A[:, c["vacc"]]
     pend.lay, pend.fslab, pend.islab, pend.tape = lay, fslab, islab, tape
     pend.seq0, pend.slot0, pend.bmat, pend.launches = seq0, slot0, bmat, launches
+    pend.zero_bwd = zero is not None and bmat is not None and not _zero_in_forward()
     return pend
 
 
@@ -800,6 +805,7 @@ def _collect_frames(pend: _Pending) -> BatchResult:
     if bmat is not None:
         bmat[:, _BC["n_verts"]:_BC["n_quad_tets"] + 1] = sizes[:, (4, 1, 2)]
     res = BatchResult(frames, fslab, islab, pend.tape, lay.tape_off, launches, bmat)
+    res.zero_bwd = pend.zero_bwd
     res.geom = (cv, cfa, i_len)      # cap_v, cap_fa, int64 words per frame of the index slab (tangent branch of the backward)
     return res
 
@@ -911,10 +917,33 @@ def _ref_arrays(refs, need):
     return out
 
 
+def _zero_in_forward() -> bool:
+    """D3H_ZERO_IN_FORWARD=1: the forward call zero-fills the dense gradient buffers (next to its surface kernels)
+    instead of the backward call.  The default is the backward call: the forward rounds of a training step are its
+    critical path, while the GPU waits for the host around the backward call; the switch keeps both placements
+    measurable."""
+    return os.environ.get("D3H_ZERO_IN_FORWARD") == "1"
+
+
+def _zero_backward(bmat, stream) -> None:
+    """Zero-fills the gradient buffers of a batch ahead of its adjoints: ONE d3h_extract_backward_batch call with the
+    batch's blocks, grads_prezeroed = 0 and no upstream gradients -- the library launches its zero-fill (every buffer
+    once, however many frames share it) and no adjoint.  The adjoint call that follows passes grads_prezeroed = 1, so a
+    buffer the frames share is never zeroed between two frames' contributions."""
+    z = bmat.copy()
+    b = _BC
+    z[:, b["g_verts_aug"]:b["g_msdf_wt"] + 1] = 0
+    z[:, b["g_msdf_boundary"]] = z[:, b["g_verts_tng"]] = z[:, b["g_mvert_tng"]] = 0
+    z[:, b["grads_prezeroed"]] &= 0xFFFFFFFF          # grads_prezeroed = 0 (the high half of the word)
+    _cabi.check(_cabi.lib().d3h_extract_backward_batch(z.ctypes.data, z.shape[0], 1, stream), "d3h_extract_backward_batch")
+    _ExtractFn.total_launches += 1
+
+
 def _prelaunch(refs, tensors, need, tets_i32, watertight_template, lanes, launcher=None, static=None, fused_pair=False):
     """Everything of a forward call that precedes the size read: pointer tables of the frames, dense gradient buffers
-    (allocated here, zero-filled by the tail of the forward call of the frame that owns them -- HBM is idle behind the
-    latency-bound surface kernels), and the launch.  Returns (pending batch, gradient buffers or None, N)."""
+    (allocated here, uninitialised: the backward call zero-fills them before its adjoints -- or, with
+    D3H_ZERO_IN_FORWARD=1, the forward call of the frame that owns them), and the launch.
+    Returns (pending batch, gradient buffers or None, N)."""
     need = tuple(bool(x) for x in need)
     idx, row, neg, gmask, zmask, used = _ref_arrays(refs, need)
     n_grid = tensors[refs[0][0][0]].shape[-2]
@@ -961,7 +990,7 @@ class _ExtractFn(torch.autograd.Function):
         res = _collect_frames(pend)
         ctx.save_for_backward(*tensors, res.tape, res.fslab)   # the slabs hold the tape and verts_wt / msdf_wt of all frames
         ctx.islab = res.islab                                  # faces_watertight: only read by the tangent branch of the backward pass
-        ctx.bmat = res.bmat
+        ctx.bmat, ctx.zero_bwd = res.bmat, res.zero_bwd
         ctx.meta = (refs, tets_i32.shape[0], n_grid, [(f.n_verts, f.n_tri, f.n_quad) for f in res.frames], lanes)
         ctx.caps = res.geom
         ctx.gbufs = gbufs
@@ -984,7 +1013,7 @@ class _ExtractFn(torch.autograd.Function):
         refs, n_tets, n_grid, sizes, lanes = ctx.meta
         tensors = ctx.saved_tensors[:-2]
         need = ctx.needs_input_grad[2:]
-        gbufs, ctx.gbufs = ctx.gbufs, None       # the pre-zeroed buffers serve ONE backward pass
+        gbufs, ctx.gbufs = ctx.gbufs, None       # the forward call's buffers serve ONE backward pass
         bmat = ctx.bmat
         if bmat is None:
             raise RuntimeError("backward through an extraction whose inputs did not require gradients")
@@ -1004,6 +1033,8 @@ class _ExtractFn(torch.autograd.Function):
                         if gbufs[idx] is None:
                             gbufs[idx] = torch.zeros_like(tensors[idx])
                         bmat[i, _BC[names[k]]] = gbufs[idx].data_ptr() + (row * row_bytes[k] if row > 0 else 0)
+            elif ctx.zero_bwd:
+                _zero_backward(bmat, torch.cuda.current_stream(dev).cuda_stream)
             keep = []
             live = []
             tng = []  # frames with upstream tangent gradients: (frame, g_verts, g_mvert, kept tensors)
@@ -1297,6 +1328,7 @@ class _PackedFn(torch.autograd.Function):
                 ast(islab, (B, cfa, 3), (il, 3, 1), 0), ast(islab, (B, cfw, 3), (il, 3, 1), 3 * cfa))
         ctx.save_for_backward(*tensors, pend.tape, fslab)
         ctx.bmat, ctx.gbufs, ctx.sizes, ctx.lanes, ctx.nref = pend.bmat, gbufs, sizes, lanes, len(refs)
+        ctx.zero_bwd = pend.zero_bwd
         ctx.set_materialize_grads(False)
         ctx.mark_non_differentiable(outs[6], outs[7])
         _ExtractFn.last_counts = None
@@ -1318,6 +1350,10 @@ class _PackedFn(torch.autograd.Function):
             raise RuntimeError("backward through a packed batch needs inputs that require gradients, and runs once "
                                "(use extract_frames for retain_graph)")
         B = ctx.nref
+        dev = tensors[0].device
+        if ctx.zero_bwd:
+            with torch.cuda.device(dev):
+                _zero_backward(bmat, torch.cuda.current_stream(dev).cuda_stream)
         if g0 is None and g2 is None and g3 is None and g5 is None:
             return (None, None) + tuple(gbufs[i] if need[i] else None for i in range(len(tensors)))
         keep = []
@@ -1338,7 +1374,6 @@ class _PackedFn(torch.autograd.Function):
         bmat[:, b["g_verts_wt"]] = ptrs(g3, (3, 1))
         bmat[:, b["g_msdf_wt"]] = ptrs(g5, (1,))
         bmat[:, b["g_msdf_boundary"]] = 0
-        dev = tensors[0].device
         per16 = 2 if int(bmat[0, b["tape_slots"]]) == 0 else 1
         _ExtractFn.total_launches += per16 * ((B + 15) // 16)
         with torch.cuda.device(dev):

@@ -100,8 +100,9 @@ typedef struct d3h_forward_args {
   int32_t* tape_slots;     /* (4*cap_valid_tets) corner slots grouped by watertight vertex (the sorted inverse map);
                               general path only: not written when edge_off is given */
   int32_t* tape_runs;      /* (cap_verts + 1) start of every vertex's run in tape_slots; [V] = P; general path only */
-  /* optional: dense gradient buffers of the coming backward call, zero-filled here while the latency-bound surface
-   * stages leave HBM idle (pass them to d3h_extract_backward with grads_prezeroed = 1); NULL = not wanted */
+  /* optional: dense gradient buffers of the coming backward call, zero-filled here next to the latency-bound surface
+   * stages (pass them to d3h_extract_backward with grads_prezeroed = 1); NULL = not wanted: the backward call zeroes
+   * them instead (grads_prezeroed = 0) */
   float* zero_g_pos;       /* (N,3) */
   float* zero_g_sdf;       /* (N)   */
   float* zero_g_msdf;      /* (N)   */
@@ -200,7 +201,8 @@ typedef struct d3h_backward_args {
   const float* msdf;
   int64_t n_grid;
   int32_t msdf_negate;
-  int32_t grads_prezeroed; /* 1: g_pos / g_sdf / g_msdf were zero-filled by the forward call (zero_g_*) */
+  int32_t grads_prezeroed; /* 1: g_pos / g_sdf / g_msdf are zero on entry (the forward call filled them, zero_g_*);
+                              0: the backward call zeroes them before it accumulates */
   /* saved by forward */
   const int32_t* tape_edges;
   const int32_t* tape_corners;
@@ -298,8 +300,10 @@ int d3h_extract_backward(const d3h_backward_args* args, d3h_stream_t stream);
  *   forward : args[i] as for d3h_extract_forward; frames on different lanes need distinct workspaces (frames of the same
  *             lane may share one); every frame publishes its own counts (args[i].counts_host, args[i].seq).
  *   backward: gradient buffers may be shared between frames (sdf / msdf common to all frames): all frames accumulate
- *             with atomics, a shared buffer must be zero on entry (grads_prezeroed = 1).  The adjoints of up to 16
- *             frames are one kernel launch (grid.y = frame); `lanes` is ignored. */
+ *             with atomics.  The buffers of the frames with grads_prezeroed = 0 are zeroed first, in one launch, a
+ *             shared buffer once; with grads_prezeroed = 1 on every frame that uses it, a buffer must be zero on entry.
+ *             Frames without a surface or without upstream gradients are zeroed too and otherwise skipped.  The
+ *             adjoints of up to 16 consecutive frames are one kernel launch (grid.y = frame); `lanes` is ignored. */
 int d3h_extract_forward_batch(const d3h_forward_args* args, int64_t n_frames, int32_t lanes, d3h_stream_t stream);
 /* The same without the final join: `stream` is not ordered behind the lanes until d3h_lanes_join(stream).  Batches
  * launched back to back this way queue up per lane (no drain / refill of the lanes at the batch boundary); the caller

@@ -1,13 +1,15 @@
 #!/usr/bin/env bash
 # A/B of this tree against another build of the project (PARENT=<its root>, built), in one session on one GPU:
 #   the GPU suite and smoke() of this tree, bench.py alternating between the two builds, the output dumps of both compared
-#   (profiles/compare_dumps.py, with a second dump of the parent for the run-to-run spread of the float atomics) and one
-#   step timeline per build.  Everything lands under OUT=<directory>.
+#   (profiles/compare_dumps.py, with a second dump of the parent for the run-to-run spread of the float atomics) and the
+#   step timelines of one and of two groups per build.  ARMS adds arms that run this tree with extra environment, e.g.
+#   ARMS="fwd:D3H_ZERO_IN_FORWARD=1".  Everything lands under OUT=<directory>.
 set -u
 cd "$(dirname "$0")/.."
 NEW=$(pwd)
 PARENT=$(cd "${PARENT:?set PARENT to the root of the other build}" && pwd)
 RUNS=${RUNS:-3}
+ARMS=${ARMS:-}
 mkdir -p "${OUT:?set OUT to the directory for the results}"
 OUT=$(cd "$OUT" && pwd)
 BENCH_FLAGS="--no-e2e --no-cold --no-cpu-baseline --no-torch-baseline --no-sdf-query --no-lbs-stage --no-mesh-stage"
@@ -19,9 +21,10 @@ echo "== smoke"
 timeout 300 python -c "import __graft_entry__ as g; g.smoke()" 2>&1 | tail -1
 echo "== bench, alternating parent / new"
 for r in $(seq 1 "$RUNS"); do
-  for arm in parent new; do
-    root=$PARENT; [ "$arm" = new ] && root=$NEW
-    (cd "$root" && timeout 600 python bench.py $BENCH_FLAGS) > "$OUT/ab_bench_${arm}_${r}.json" 2> "$OUT/ab_bench_${arm}_${r}.err"
+  for spec in parent new $ARMS; do
+    arm=${spec%%:*}; envs=""; [ "$spec" != "$arm" ] && envs=${spec#*:}
+    root=$PARENT; [ "$arm" != parent ] && root=$NEW
+    (cd "$root" && env $envs timeout 600 python bench.py $BENCH_FLAGS) > "$OUT/ab_bench_${arm}_${r}.json" 2> "$OUT/ab_bench_${arm}_${r}.err"
     python - "$OUT/ab_bench_${arm}_${r}.json" "$arm" <<'PY'
 import json, sys
 d = json.loads(open(sys.argv[1]).read().strip().splitlines()[-1])
@@ -36,8 +39,10 @@ echo "== output dumps"
 (cd "$NEW" && timeout 600 python bench.py $BENCH_FLAGS --steps 20 --dump-outputs "$OUT/dump_new") > /dev/null 2> "$OUT/dump_new.err"
 python profiles/compare_dumps.py "$OUT/dump_parent" "$OUT/dump_new" "$OUT/dump_parent2" | tee "$OUT/ab_compare_dumps.txt"
 rm -rf "$OUT/dump_parent" "$OUT/dump_parent2" "$OUT/dump_new"
-echo "== step timelines (one group)"
-(cd "$PARENT" && NGROUPS=1 timeout 300 python profiles/step_timeline.py) > "$OUT/ab_timeline_parent.txt" 2>&1
-(cd "$NEW" && NGROUPS=1 timeout 300 python profiles/step_timeline.py) > "$OUT/ab_timeline_new.txt" 2>&1
-grep -v "Warn\|warn" "$OUT/ab_timeline_parent.txt" | grep "poly_\|step" | cut -c1-60
-grep -v "Warn\|warn" "$OUT/ab_timeline_new.txt" | grep "poly_\|step" | cut -c1-60
+echo "== step timelines (one group, two groups)"
+for g in 1 2; do
+  (cd "$PARENT" && NGROUPS=$g timeout 300 python profiles/step_timeline.py) > "$OUT/ab_timeline_${g}g_parent.txt" 2>&1
+  (cd "$NEW" && NGROUPS=$g timeout 300 python profiles/step_timeline.py) > "$OUT/ab_timeline_${g}g_new.txt" 2>&1
+  grep -v "Warn\|warn" "$OUT/ab_timeline_${g}g_parent.txt" | grep "zero\|adjoint\|step" | cut -c1-60
+  grep -v "Warn\|warn" "$OUT/ab_timeline_${g}g_new.txt" | grep "zero\|adjoint\|step" | cut -c1-60
+done
