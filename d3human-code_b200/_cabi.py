@@ -174,7 +174,7 @@ def lib() -> C.CDLL:
         L.d3h_mlp_head.argtypes = [vp, i64, i64, i32, vp, vp, i32, vp, vp]
         L.d3h_mlp_head_backward.restype = C.c_int
         L.d3h_mlp_head_backward.argtypes = [vp, i64, i64, i32, vp, i32, vp, vp, i64, vp, vp, vp]
-    # include/d3h_lbs.h (not part of the CPU emulation either)
+    # include/d3h_lbs.h (the CPU emulation of tests/emu has it too)
     if hasattr(L, "d3h_lbs_apply"):
         vp, i64, i32 = C.c_void_p, C.c_int64, C.c_int32
         L.d3h_lbs_blend.restype = C.c_int

@@ -202,21 +202,23 @@ __global__ void __launch_bounds__(256) lbs_apply_kernel(const float* __restrict_
 }
 
 // Zero rows (the bulk of verts_aug) all hit the same table row: their share of g_b is (sum of their upstream gradients)
-// (x) [can_0; 1], reduced per CTA in shared memory instead of through 12 atomics per point on one address.
+// (x) [can_0; 1], reduced per CTA in shared memory instead of through 12 atomics per point on one address.  The first zero
+// row to claim s_zero_v names the CTA's table row; a zero row with another idx (possible through the ABI, never from
+// d3h_lbs_nearest on the same points) takes the per-row atomics like a live row.
 __global__ void __launch_bounds__(256) lbs_apply_backward_kernel(const float* __restrict__ g, int64_t n, const int32_t* __restrict__ idx,
                                                                  const float* __restrict__ binv, const float* __restrict__ bpose,
                                                                  const float* __restrict__ can, const float* __restrict__ pts,
                                                                  float* __restrict__ g_pts, float* __restrict__ g_b,
                                                                  float* __restrict__ g_trans) {
-  __shared__ float s_zero[3];     // sum of g over this CTA's zero rows (pts row exactly (0,0,0))
+  __shared__ float s_zero[3];     // sum of g over this CTA's zero rows (pts row exactly (0,0,0)) with idx == s_zero_v
   __shared__ float s_all[3];      // sum of g over all rows of the CTA
-  __shared__ float s_can[3];      // canonical point of the zero rows (the same for all of them)
+  __shared__ float s_can[3];      // canonical point of those zero rows (the same for all of them: it depends on idx only)
   __shared__ int s_zero_v;
   if (threadIdx.x < 3) { s_zero[threadIdx.x] = 0.f; s_all[threadIdx.x] = 0.f; }
   if (threadIdx.x == 0) s_zero_v = -1;
   __syncthreads();
   const int64_t p = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  float gx = 0.f, gy = 0.f, gz = 0.f;
+  float gx = 0.f, gy = 0.f, gz = 0.f, cx = 0.f, cy = 0.f, cz = 0.f;
   bool zero_row = false;
   int v = 0;
   if (p < n) {
@@ -236,17 +238,19 @@ __global__ void __launch_bounds__(256) lbs_apply_backward_kernel(const float* __
       }
     }
     g_pts[3 * p] = out[0]; g_pts[3 * p + 1] = out[1]; g_pts[3 * p + 2] = out[2];
-    const float cx = can[3 * p], cy = can[3 * p + 1], cz = can[3 * p + 2];
+    cx = can[3 * p]; cy = can[3 * p + 1]; cz = can[3 * p + 2];
     zero_row = pts != nullptr && pts[3 * p] == 0.f && pts[3 * p + 1] == 0.f && pts[3 * p + 2] == 0.f;
-    if (zero_row) { s_zero_v = v; s_can[0] = cx; s_can[1] = cy; s_can[2] = cz; }     // (every zero row stores the same values)
-    if (!zero_row && (gx != 0.f || gy != 0.f || gz != 0.f)) {
-      float* row = g_b + 12ll * v;
-      atomicAdd(row + 0, gx * cx); atomicAdd(row + 1, gx * cy); atomicAdd(row + 2, gx * cz); atomicAdd(row + 3, gx);
-      atomicAdd(row + 4, gy * cx); atomicAdd(row + 5, gy * cy); atomicAdd(row + 6, gy * cz); atomicAdd(row + 7, gy);
-      atomicAdd(row + 8, gz * cx); atomicAdd(row + 9, gz * cy); atomicAdd(row + 10, gz * cz); atomicAdd(row + 11, gz);
-    }
+    if (zero_row && atomicCAS(&s_zero_v, -1, v) == -1) { s_can[0] = cx; s_can[1] = cy; s_can[2] = cz; }
   }
-  // CTA sums: all rows (translation gradient) and zero rows
+  __syncthreads();
+  zero_row = zero_row && v == s_zero_v;
+  if (p < n && !zero_row && (gx != 0.f || gy != 0.f || gz != 0.f)) {
+    float* row = g_b + 12ll * v;
+    atomicAdd(row + 0, gx * cx); atomicAdd(row + 1, gx * cy); atomicAdd(row + 2, gx * cz); atomicAdd(row + 3, gx);
+    atomicAdd(row + 4, gy * cx); atomicAdd(row + 5, gy * cy); atomicAdd(row + 6, gy * cz); atomicAdd(row + 7, gy);
+    atomicAdd(row + 8, gz * cx); atomicAdd(row + 9, gz * cy); atomicAdd(row + 10, gz * cz); atomicAdd(row + 11, gz);
+  }
+  // CTA sums: all rows (translation gradient) and the zero rows of s_zero_v
   float all[3] = {gx, gy, gz}, zr[3] = {zero_row ? gx : 0.f, zero_row ? gy : 0.f, zero_row ? gz : 0.f};
 #pragma unroll
   for (int c = 0; c < 3; ++c) {
@@ -296,7 +300,12 @@ extern "C" int d3h_lbs_blend(const float* lbs_weights, const float* a, int64_t n
     return D3H_E_BADARG;
   }
   if (n_template == 0) return D3H_OK;
+#ifndef D3H_CPU_EMU
   lbs_blend_kernel<<<(unsigned)((n_template + 127) / 128), 128, 0, (cudaStream_t)stream>>>(lbs_weights, a, n_template, n_joints, invert, out);
+#else   // tests/emu: g++ has no <<< >>>
+  launch_k(lbs_blend_kernel, (unsigned)((n_template + 127) / 128), 128u, (cudaStream_t)stream, kLaunchStream, lbs_weights, a, n_template,
+           n_joints, invert, out);
+#endif
   return lbs_done("d3h_lbs_blend");
 }
 
@@ -306,7 +315,11 @@ extern "C" int d3h_lbs_blend_backward(const float* lbs_weights, const float* g_b
     set_error("d3h_lbs_blend_backward: bad argument");
     return D3H_E_BADARG;
   }
+#ifndef D3H_CPU_EMU
   lbs_blend_backward_kernel<<<(unsigned)n_joints, 256, 0, (cudaStream_t)stream>>>(lbs_weights, g_b, n_template, n_joints, g_a);
+#else
+  launch_k(lbs_blend_backward_kernel, (unsigned)n_joints, 256u, (cudaStream_t)stream, kLaunchStream, lbs_weights, g_b, n_template, n_joints, g_a);
+#endif
   return lbs_done("d3h_lbs_blend_backward");
 }
 
@@ -326,22 +339,33 @@ extern "C" int d3h_lbs_nearest(const float* pts, int64_t n_points, const float* 
   ws.list = ws.count + 16;
   cudaMemsetAsync(ws.count, 0, 64, st);
   const unsigned blocks = (unsigned)((n_points + 255) / 256);
+#ifndef D3H_CPU_EMU
   lbs_compact_kernel<<<blocks, 256, 0, st>>>(pts, n_points, ws);
   lbs_nearest_kernel<<<(unsigned)((n_points + 1 + 255) / 256), 256, 0, st>>>(pts, tmpl, n_template, ws, idx);
   lbs_fill_zero_kernel<<<blocks, 256, 0, st>>>(pts, n_points, ws, idx);
+#else
+  launch_k(lbs_compact_kernel, blocks, 256u, st, kLaunchStream, pts, n_points, ws);
+  launch_k(lbs_nearest_kernel, (unsigned)((n_points + 1 + 255) / 256), 256u, st, kLaunchStream, pts, tmpl, n_template, ws, idx);
+  launch_k(lbs_fill_zero_kernel, blocks, 256u, st, kLaunchStream, pts, n_points, ws, idx);
+#endif
   return lbs_done("d3h_lbs_nearest");
 }
 
 extern "C" int d3h_lbs_apply(const float* pts, int64_t n_points, const int32_t* idx, const float* b_init_inv, const float* b_pose,
                              const float* trans, float* canonical, float* posed, d3h_stream_t stream) {
-  if (n_points < 0 || !b_init_inv || !al16(b_init_inv) || !al16(b_pose) || (b_pose && !posed) ||
-      (n_points > 0 && (!pts || !idx || !canonical))) {
+  if (n_points < 0 || !b_init_inv || !al16(b_init_inv) || !al16(b_pose) ||
+      (n_points > 0 && (!pts || !idx || !canonical || (b_pose && !posed)))) {
     set_error("d3h_lbs_apply: bad argument (tables 16-byte aligned; posed required with b_pose)");
     return D3H_E_BADARG;
   }
   if (n_points == 0) return D3H_OK;
+#ifndef D3H_CPU_EMU
   lbs_apply_kernel<<<(unsigned)((n_points + 255) / 256), 256, 0, (cudaStream_t)stream>>>(pts, n_points, idx, b_init_inv, b_pose, trans,
                                                                                      canonical, posed);
+#else
+  launch_k(lbs_apply_kernel, (unsigned)((n_points + 255) / 256), 256u, (cudaStream_t)stream, kLaunchStream, pts, n_points, idx, b_init_inv,
+           b_pose, trans, canonical, posed);
+#endif
   return lbs_done("d3h_lbs_apply");
 }
 
@@ -354,7 +378,12 @@ extern "C" int d3h_lbs_apply_backward(const float* g_posed, int64_t n_points, co
     return D3H_E_BADARG;
   }
   if (n_points == 0) return D3H_OK;
+#ifndef D3H_CPU_EMU
   lbs_apply_backward_kernel<<<(unsigned)((n_points + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
       g_posed, n_points, idx, b_init_inv, b_pose, canonical, pts, g_pts, g_b, g_trans);
+#else
+  launch_k(lbs_apply_backward_kernel, (unsigned)((n_points + 255) / 256), 256u, (cudaStream_t)stream, kLaunchStream, g_posed, n_points, idx,
+           b_init_inv, b_pose, canonical, pts, g_pts, g_b, g_trans);
+#endif
   return lbs_done("d3h_lbs_apply_backward");
 }

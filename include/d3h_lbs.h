@@ -50,7 +50,9 @@ int d3h_lbs_apply(const float* pts, int64_t n_points, const int32_t* idx, const 
  *   g_b[v]    += sum over the points with idx[p] = v of g_posed[p] (x) [can[p];1]   (Vt,12: the first three rows of B_pose)
  *   g_trans   += sum_p g_posed[p]                                              (3), may be NULL
  * g_b / g_trans ACCUMULATE (zero them first).  `pts` (the forward input, may be NULL) lets the kernel sum the upstream
- * gradients of the all-zero rows per CTA instead of through twelve atomics per row on one table row. */
+ * gradients of the all-zero rows per CTA instead of through twelve atomics per row on one table row.  The zero rows need
+ * not share one idx: per CTA the zero rows of one idx are summed, the others take the per-row atomics.  The result is the
+ * same as with pts == NULL up to the order of the float additions. */
 int d3h_lbs_apply_backward(const float* g_posed, int64_t n_points, const int32_t* idx, const float* b_init_inv,
                            const float* b_pose, const float* canonical, const float* pts, float* g_pts, float* g_b,
                            float* g_trans, d3h_stream_t stream);

@@ -36,9 +36,10 @@ def blend(lbs_weights, A):
     return np.einsum("vj,jab->vab", np.asarray(lbs_weights, np.float64), np.asarray(A, np.float64))
 
 
-def lbs_forward(pts, template, lbs_weights, init_A, A, trans):
-    """deformer.lbs_forward :472-476 for one frame.  -> (posed (P,3), cache)"""
-    idx = nearest(pts, template)
+def lbs_forward(pts, template, lbs_weights, init_A, A, trans, idx=None):
+    """deformer.lbs_forward :472-476 for one frame.  -> (posed (P,3), cache).  idx (P): nearest template vertex of every
+    point when already known (None: searched here)"""
+    idx = nearest(pts, template) if idx is None else np.asarray(idx, np.int64)
     b_init, b_pose = blend(lbs_weights, init_A), blend(lbs_weights, A)
     inv = np.linalg.inv(b_init)
     ph = np.concatenate([np.asarray(pts, np.float64), np.ones((len(pts), 1))], 1)
@@ -48,9 +49,9 @@ def lbs_forward(pts, template, lbs_weights, init_A, A, trans):
     return posed, dict(idx=idx, inv=inv, b_pose=b_pose, can_h=ch, lbs_weights=np.asarray(lbs_weights, np.float64))
 
 
-def lbs_forward_inverse(pts, template, lbs_weights, init_A):
+def lbs_forward_inverse(pts, template, lbs_weights, init_A, idx=None):
     """deformer.lbs_forward_inverse :424-430"""
-    idx = nearest(pts, template)
+    idx = nearest(pts, template) if idx is None else np.asarray(idx, np.int64)
     inv = np.linalg.inv(blend(lbs_weights, init_A))
     ph = np.concatenate([np.asarray(pts, np.float64), np.ones((len(pts), 1))], 1)
     return np.einsum("pab,pb->pa", inv[idx], ph)[:, :3]

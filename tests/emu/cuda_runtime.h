@@ -177,6 +177,8 @@ static inline int min(int a, int b) { return a < b ? a : b; }
 static inline int max(int a, int b) { return a > b ? a : b; }
 static inline unsigned min(unsigned a, unsigned b) { return a < b ? a : b; }
 static inline unsigned max(unsigned a, unsigned b) { return a > b ? a : b; }
+static inline long min(long a, long b) { return a < b ? a : b; }   // int64_t is long on LP64: min(int64_t, int64_t)
+static inline long max(long a, long b) { return a > b ? a : b; }
 static inline long long min(long long a, long long b) { return a < b ? a : b; }
 static inline long long max(long long a, long long b) { return a > b ? a : b; }
 
@@ -224,6 +226,10 @@ static inline unsigned atomicCAS(unsigned* p, unsigned cmp, unsigned v) {
   __atomic_compare_exchange_n(p, &cmp, v, false, __ATOMIC_SEQ_CST, __ATOMIC_SEQ_CST);
   return cmp;
 }
+static inline int atomicCAS(int* p, int cmp, int v) {
+  __atomic_compare_exchange_n(p, &cmp, v, false, __ATOMIC_SEQ_CST, __ATOMIC_SEQ_CST);
+  return cmp;
+}
 static inline unsigned long long atomicMax(unsigned long long* p, unsigned long long v) {
   unsigned long long old = __atomic_load_n(p, __ATOMIC_RELAXED);
   while (old < v && !__atomic_compare_exchange_n(p, &old, v, false, __ATOMIC_SEQ_CST, __ATOMIC_RELAXED)) {}
@@ -242,6 +248,11 @@ static inline unsigned long long atomicCAS(unsigned long long* p, unsigned long 
 }
 static inline unsigned atomicCAS(unsigned* p, unsigned cmp, unsigned v) {
   unsigned o = *p;
+  if (o == cmp) *p = v;
+  return o;
+}
+static inline int atomicCAS(int* p, int cmp, int v) {
+  int o = *p;
   if (o == cmp) *p = v;
   return o;
 }
