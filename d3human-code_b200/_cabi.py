@@ -25,6 +25,8 @@ EXPORTED_SYMBOLS = (
     "d3h_lbs_blend", "d3h_lbs_blend_backward", "d3h_lbs_nearest_workspace_bytes", "d3h_lbs_nearest", "d3h_lbs_apply",
     "d3h_lbs_apply_backward",
     "d3h_mlp_embed", "d3h_mlp_embed_backward", "d3h_mlp_packed_weight_bytes", "d3h_mlp_pack_weight", "d3h_mlp_linear", "d3h_mlp_wgrad_workspace_bytes", "d3h_mlp_wgrad", "d3h_mlp_head", "d3h_mlp_head_backward",
+    "d3h_mlp_embed_tangent", "d3h_mlp_embed_second_backward", "d3h_mlp_linear_tangent", "d3h_mlp_linear_adjoint",
+    "d3h_mlp_head_second_backward",
     "d3h_profile_enable", "d3h_profile_kinds", "d3h_profile_kernel_name", "d3h_profile_read", "d3h_profile_timeline", "d3h_profile_scan_kernel", "d3h_trace_enable", "d3h_trace_read", "d3h_debug_table",
 )
 
@@ -174,6 +176,16 @@ def lib() -> C.CDLL:
         L.d3h_mlp_head.argtypes = [vp, i64, i64, i32, vp, vp, i32, vp, vp]
         L.d3h_mlp_head_backward.restype = C.c_int
         L.d3h_mlp_head_backward.argtypes = [vp, i64, i64, i32, vp, i32, vp, vp, i64, vp, vp, vp]
+        L.d3h_mlp_embed_tangent.restype = C.c_int
+        L.d3h_mlp_embed_tangent.argtypes = [vp, vp, i64, i32, vp, i64, i32, vp]
+        L.d3h_mlp_embed_second_backward.restype = C.c_int
+        L.d3h_mlp_embed_second_backward.argtypes = [vp, vp, i64, i32, vp, i64, vp, i64, vp, vp]
+        L.d3h_mlp_linear_tangent.restype = C.c_int
+        L.d3h_mlp_linear_tangent.argtypes = [vp, i64, i64, i32, vp, i32, vp, i64, vp, i64, vp, i64, vp]
+        L.d3h_mlp_linear_adjoint.restype = C.c_int
+        L.d3h_mlp_linear_adjoint.argtypes = [vp, i64, i64, i32, vp, i32, vp, i64, vp, i64, vp, i64, vp, i64, vp]
+        L.d3h_mlp_head_second_backward.restype = C.c_int
+        L.d3h_mlp_head_second_backward.argtypes = [vp, i64, vp, i64, vp, i64, vp, i64, i64, i32, vp, i32, vp, vp, i64, vp]
     # include/d3h_lbs.h (the CPU emulation of tests/emu has it too)
     if hasattr(L, "d3h_lbs_apply"):
         vp, i64, i32 = C.c_void_p, C.c_int64, C.c_int32

@@ -19,6 +19,8 @@
 //     apply bias / Softplus(beta=100) / the activation's derivative, and store fp32 rows.
 //
 // mlp_linear_kernel : c = f(a w^T + bias), tile = 128 rows of a x all N <= 256 output columns, K walked in 32-column slices.
+//                     Two more epilogues serve the second derivative (the eikonal term): tangent (z-dot and a-dot =
+//                     z-dot * softplus') and adjoint (input gradient * softplus' + the softplus'' term of delta and z-dot).
 // mlp_wgrad_kernel  : dw += dz^T a, the contraction runs over the POINTS: the producers transpose 32-point slices of dz
 //                     and a on their way into shared memory (lanes <-> points, conflict-free), every CTA owns a point
 //                     range and 128 of dz's columns and adds its partial result to dw with red.global.add.f32.
@@ -159,6 +161,11 @@ __device__ __forceinline__ float softplus100(float z) {
 // d softplus / dz from the OUTPUT y = softplus(z): sigmoid(beta z) = 1 - exp(-beta y)  (exactly 1 - e^-20.. in the linear
 // branch, where torch's backward returns 1: the difference is < 2.1e-9)
 __device__ __forceinline__ float softplus100_grad_from_output(float y) { return 1.f - __expf(-kBeta * y); }
+// softplus''(z) / softplus'(z) = beta (1 - softplus'(z)) = beta exp(-beta y), zero past the threshold as in torch's
+// softplus_double_backward: the factor that turns delta = lambda softplus'(z) into lambda softplus''(z)
+__device__ __forceinline__ float softplus100_curv_from_output(float y) {
+  return kBeta * y <= kThreshold ? kBeta * __expf(-kBeta * y) : 0.f;
+}
 
 struct StageBuffers {       // byte offsets inside the dynamic shared memory of one stage
   uint32_t a_hi, a_lo, b_hi, b_lo, bytes;
@@ -224,9 +231,18 @@ struct LinearArgs {
   float* c; int64_t ldc;
   int64_t m;
   int k, n, mode;
+  float* c2; int64_t ldc2;           // kEpiTangent: z-dot
+  const float* d; int64_t ldd;       // kEpiAdjoint: delta and z-dot of the layer whose output is y
+  const float* zd; int64_t ldzd;
 };
 
+// Epilogues of mlp_linear_kernel.  kEpiFirstOrder: `mode` 0 / 1 / 2 of d3h_mlp_linear.  The other two serve the second
+// derivative (d3h_mlp_linear_tangent / d3h_mlp_linear_adjoint): tangent c2 = acc, c = acc * softplus'(y); adjoint
+// c = acc * softplus'(y) + beta [beta y <= 20] exp(-beta y) * d * zd.
+constexpr int kEpiFirstOrder = 0, kEpiTangent = 1, kEpiAdjoint = 2;
+
 // ---------------------------------------------------------------------------------------------- c = f(a w^T + bias)
+template <int kEpi>
 __global__ void __launch_bounds__(kThreads, kCtasPerSm) mlp_linear_kernel(LinearArgs g) {
   extern __shared__ __align__(1024) uint8_t smem[];
   __shared__ uint64_t s_full, s_empty, s_done;
@@ -297,7 +313,25 @@ __global__ void __launch_bounds__(kThreads, kCtasPerSm) mlp_linear_kernel(Linear
     for (int c0 = half * ncol_half; c0 < (half + 1) * ncol_half; c0 += 32) {
       float v[32];
       tmem_ld32(tmem_d + ((uint32_t)(32 * q) << 16) + (uint32_t)c0, v);
-      if (r < g.m) {
+      if (kEpi != kEpiFirstOrder && r < g.m) {
+#pragma unroll
+        for (int j = 0; j < 32; j += 4) {
+          const float4 yy = __ldg(reinterpret_cast<const float4*>(g.y + r * g.ldy + c0 + j));
+          const float4 acc = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
+          float4 o = make_float4(acc.x * softplus100_grad_from_output(yy.x), acc.y * softplus100_grad_from_output(yy.y),
+                                 acc.z * softplus100_grad_from_output(yy.z), acc.w * softplus100_grad_from_output(yy.w));
+          if (kEpi == kEpiTangent) {
+            *reinterpret_cast<float4*>(g.c2 + r * g.ldc2 + c0 + j) = acc;
+          } else {
+            const float4 dd = __ldg(reinterpret_cast<const float4*>(g.d + r * g.ldd + c0 + j));
+            const float4 zz = __ldg(reinterpret_cast<const float4*>(g.zd + r * g.ldzd + c0 + j));
+            o.x += softplus100_curv_from_output(yy.x) * dd.x * zz.x; o.y += softplus100_curv_from_output(yy.y) * dd.y * zz.y;
+            o.z += softplus100_curv_from_output(yy.z) * dd.z * zz.z; o.w += softplus100_curv_from_output(yy.w) * dd.w * zz.w;
+          }
+          *reinterpret_cast<float4*>(g.c + r * g.ldc + c0 + j) = o;
+        }
+      }
+      if (kEpi == kEpiFirstOrder && r < g.m) {
 #pragma unroll
         for (int j = 0; j < 32; j += 4) {
           float o[4];
@@ -646,6 +680,100 @@ __global__ void __launch_bounds__(256) head_backward_kernel(const float* __restr
   if (db != nullptr && threadIdx.x < DOUT) atomicAdd(db + threadIdx.x, s_db[0][threadIdx.x] + s_db[1][threadIdx.x] + s_db[2][threadIdx.x] + s_db[3][threadIdx.x]);
 }
 
+// ---------------------------------------------------------------------------------------------- second derivative
+// Directional derivative of the encoding along v: out = [v, 2^k cos(2^k x) v, -2^k sin(2^k x) v, ...], zero padding up to
+// n_cols.  One thread per point (the GEMMs that read it dominate).
+__global__ void __launch_bounds__(256) embed_tangent_kernel(const float* __restrict__ x, const float* __restrict__ v, int64_t m,
+                                                            int n_freq, float* __restrict__ out, int64_t ld, int n_cols) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= m) return;
+  const float p[3] = {x[3 * i], x[3 * i + 1], x[3 * i + 2]};
+  const float t[3] = {v[3 * i], v[3 * i + 1], v[3 * i + 2]};
+  float* o = out + i * ld;
+  o[0] = t[0]; o[1] = t[1]; o[2] = t[2];
+  float f = 1.f;
+  for (int k = 0; k < n_freq; ++k, f *= 2.f) {
+#pragma unroll
+    for (int d = 0; d < 3; ++d) {
+      float s, c;
+      sincosf(f * p[d], &s, &c);
+      o[3 + 6 * k + d] = f * c * t[d];
+      o[6 + 6 * k + d] = -f * s * t[d];
+    }
+  }
+  for (int c = 3 * (2 * n_freq + 1); c < n_cols; ++c) o[c] = 0.f;
+}
+
+// g_x = E'(x)^T gbar + E''(x)[v]^T g_emb: the adjoint of the encoding applied to gbar (skipped when gbar is null) plus the
+// derivative of the first adjoint E'(x)^T g_emb along v, diagonal per coordinate: sum_k -4^k v (sin(2^k x) g_sin + cos(2^k x) g_cos).
+__global__ void __launch_bounds__(256) embed_second_backward_kernel(const float* __restrict__ x, const float* __restrict__ v,
+                                                                    int64_t m, int n_freq, const float* __restrict__ gbar,
+                                                                    int64_t ldbar, const float* __restrict__ g_emb, int64_t ld,
+                                                                    float* __restrict__ g_x) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= m) return;
+  const float* gb = gbar ? gbar + i * ldbar : nullptr;
+  const float* ge = g_emb + i * ld;
+  float acc[3] = {0.f, 0.f, 0.f};
+  if (gb) { acc[0] = gb[0]; acc[1] = gb[1]; acc[2] = gb[2]; }
+  float f = 1.f;
+  for (int k = 0; k < n_freq; ++k, f *= 2.f) {
+#pragma unroll
+    for (int d = 0; d < 3; ++d) {
+      float s, c;
+      sincosf(f * x[3 * i + d], &s, &c);
+      if (gb) acc[d] += f * (c * gb[3 + 6 * k + d] - s * gb[6 + 6 * k + d]);
+      acc[d] -= f * f * v[3 * i + d] * (s * ge[3 + 6 * k + d] + c * ge[6 + 6 * k + d]);
+    }
+  }
+#pragma unroll
+  for (int d = 0; d < 3; ++d) g_x[3 * i + d] = acc[d];
+}
+
+// Second derivative through the output layer in one sweep, laid out as head_backward_kernel:
+//   dw[j, k] += sum_m g[m, j] adot[m, k],   mu[m, k] = beta [beta a <= 20] exp(-beta a) delta zdot   (a, delta, zdot at m, k)
+template <int DOUT>
+__global__ void __launch_bounds__(256) head_second_backward_kernel(const float* __restrict__ adot, int64_t ldad,
+                                                                   const float* __restrict__ a, int64_t lda,
+                                                                   const float* __restrict__ delta, int64_t ldd,
+                                                                   const float* __restrict__ zdot, int64_t ldzd, int64_t m, int k,
+                                                                   const float* __restrict__ g, float* __restrict__ dw,
+                                                                   float* __restrict__ mu, int64_t ldmu) {
+  __shared__ float s_dw[4][DOUT][256];
+  const int x = threadIdx.x & 63, y = threadIdx.x >> 6;
+  const int64_t r_begin = (int64_t)blockIdx.x * kHeadRows, r_end = min(m, r_begin + kHeadRows);
+  const int groups = k / 4;
+  float4 acc[DOUT];
+#pragma unroll
+  for (int j = 0; j < DOUT; ++j) acc[j] = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (x < groups) {
+    for (int64_t r = r_begin + y; r < r_end; r += 4) {
+      const float4 ad = __ldg(reinterpret_cast<const float4*>(adot + r * ldad) + x);
+#pragma unroll
+      for (int j = 0; j < DOUT; ++j) {
+        const float gj = __ldg(g + r * DOUT + j);
+        acc[j].x = fmaf(gj, ad.x, acc[j].x); acc[j].y = fmaf(gj, ad.y, acc[j].y);
+        acc[j].z = fmaf(gj, ad.z, acc[j].z); acc[j].w = fmaf(gj, ad.w, acc[j].w);
+      }
+      const float4 av = __ldg(reinterpret_cast<const float4*>(a + r * lda) + x);
+      const float4 dv = __ldg(reinterpret_cast<const float4*>(delta + r * ldd) + x);
+      const float4 zv = __ldg(reinterpret_cast<const float4*>(zdot + r * ldzd) + x);
+      *(reinterpret_cast<float4*>(mu + r * ldmu) + x) =
+          make_float4(softplus100_curv_from_output(av.x) * dv.x * zv.x, softplus100_curv_from_output(av.y) * dv.y * zv.y,
+                      softplus100_curv_from_output(av.z) * dv.z * zv.z, softplus100_curv_from_output(av.w) * dv.w * zv.w);
+    }
+  }
+#pragma unroll
+  for (int j = 0; j < DOUT; ++j) {
+    s_dw[y][j][4 * x] = acc[j].x; s_dw[y][j][4 * x + 1] = acc[j].y; s_dw[y][j][4 * x + 2] = acc[j].z; s_dw[y][j][4 * x + 3] = acc[j].w;
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < DOUT * k; i += 256) {
+    const int j = i / k, c = i % k;
+    atomicAdd(dw + i, s_dw[0][j][c] + s_dw[1][j][c] + s_dw[2][j][c] + s_dw[3][j][c]);
+  }
+}
+
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
 }  // namespace mlp
@@ -658,6 +786,16 @@ static int finish_launch(const char* who) {
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) { set_error("%s: %s", who, cudaGetErrorString(e)); return D3H_E_CUDA; }
   return D3H_OK;
+}
+
+template <int kEpi>
+static void launch_linear(const LinearArgs& g, d3h_stream_t stream) {
+  static bool attr = false;
+  if (!attr) {
+    cudaFuncSetAttribute(mlp_linear_kernel<kEpi>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)stage_layout(256).bytes);
+    attr = true;
+  }
+  mlp_linear_kernel<kEpi><<<(unsigned)((g.m + kTileM - 1) / kTileM), kThreads, stage_layout(g.n).bytes, (cudaStream_t)stream>>>(g);
 }
 
 extern "C" int d3h_mlp_embed(const float* x, int64_t m, int32_t n_freq, float* out, int64_t ld, int32_t n_cols,
@@ -713,15 +851,102 @@ extern "C" int d3h_mlp_linear(const float* a, int64_t lda, int64_t m, int32_t k,
     return D3H_E_BADARG;
   }
   if (m == 0) return D3H_OK;
-  const size_t smem = stage_layout(n).bytes;
-  static bool attr = false;
-  if (!attr) {
-    cudaFuncSetAttribute(mlp_linear_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)stage_layout(256).bytes);
-    attr = true;
-  }
   LinearArgs g{a, lda, w_packed, bias, y, ldy, c, ldc, m, k, n, mode};
-  mlp_linear_kernel<<<(unsigned)((m + kTileM - 1) / kTileM), kThreads, smem, (cudaStream_t)stream>>>(g);
+  launch_linear<kEpiFirstOrder>(g, stream);
   return finish_launch("d3h_mlp_linear");
+}
+
+// shape / alignment rules of the tangent and adjoint variants: those of d3h_mlp_linear, with y always required
+static bool linear_shape_ok(const float* a, int64_t lda, int64_t m, int32_t k, const float* w_packed, int32_t n,
+                            const float* y, int64_t ldy, const float* c, int64_t ldc) {
+  return m >= 0 && k > 0 && (k % kSliceK) == 0 && n >= 64 && n <= 256 && (n % 64) == 0 && lda >= k && ldc >= n &&
+         (lda % 4) == 0 && (ldc % 4) == 0 && w_packed && (m == 0 || (a && c && y)) && aligned16(a) && aligned16(w_packed) &&
+         aligned16(c) && ldy >= n && (ldy % 4) == 0 && aligned16(y);
+}
+static bool operand_ok(const float* p, int64_t ld, int64_t m, int32_t n) {
+  return (m == 0 || p) && ld >= n && (ld % 4) == 0 && aligned16(p);
+}
+
+extern "C" int d3h_mlp_linear_tangent(const float* a, int64_t lda, int64_t m, int32_t k, const float* w_packed, int32_t n,
+                                      const float* y, int64_t ldy, float* zdot, int64_t ldzd, float* adot, int64_t ldad,
+                                      d3h_stream_t stream) {
+  if (!linear_shape_ok(a, lda, m, k, w_packed, n, y, ldy, adot, ldad) || !operand_ok(zdot, ldzd, m, n)) {
+    set_error("d3h_mlp_linear_tangent: bad argument (K %% 32 == 0, N in {64, 128, 192, 256}, y / zdot / adot of N columns, "
+              "leading dimensions multiples of 4, 16-byte aligned pointers)");
+    return D3H_E_BADARG;
+  }
+  if (m == 0) return D3H_OK;
+  LinearArgs g{a, lda, w_packed, nullptr, y, ldy, adot, ldad, m, k, n, 0, zdot, ldzd};
+  launch_linear<kEpiTangent>(g, stream);
+  return finish_launch("d3h_mlp_linear_tangent");
+}
+
+extern "C" int d3h_mlp_linear_adjoint(const float* a, int64_t lda, int64_t m, int32_t k, const float* w_packed, int32_t n,
+                                      const float* y, int64_t ldy, const float* delta, int64_t ldd, const float* zdot,
+                                      int64_t ldzd, float* c, int64_t ldc, d3h_stream_t stream) {
+  if (!linear_shape_ok(a, lda, m, k, w_packed, n, y, ldy, c, ldc) || !operand_ok(delta, ldd, m, n) ||
+      !operand_ok(zdot, ldzd, m, n)) {
+    set_error("d3h_mlp_linear_adjoint: bad argument (K %% 32 == 0, N in {64, 128, 192, 256}, y / delta / zdot / c of N "
+              "columns, leading dimensions multiples of 4, 16-byte aligned pointers)");
+    return D3H_E_BADARG;
+  }
+  if (m == 0) return D3H_OK;
+  LinearArgs g{a, lda, w_packed, nullptr, y, ldy, c, ldc, m, k, n, 0, nullptr, 0, delta, ldd, zdot, ldzd};
+  launch_linear<kEpiAdjoint>(g, stream);
+  return finish_launch("d3h_mlp_linear_adjoint");
+}
+
+extern "C" int d3h_mlp_embed_tangent(const float* x, const float* v, int64_t m, int32_t n_freq, float* out, int64_t ld,
+                                     int32_t n_cols, d3h_stream_t stream) {
+  if (m < 0 || n_freq < 0 || n_freq > 16 || n_cols < 3 * (2 * n_freq + 1) || ld < n_cols || (m > 0 && (!x || !v || !out))) {
+    set_error("d3h_mlp_embed_tangent: bad argument (n_cols must hold the 3 (2 n_freq + 1) channels, ld >= n_cols)");
+    return D3H_E_BADARG;
+  }
+  if (m == 0) return D3H_OK;
+  embed_tangent_kernel<<<(unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, v, m, n_freq, out, ld, n_cols);
+  return finish_launch("d3h_mlp_embed_tangent");
+}
+
+extern "C" int d3h_mlp_embed_second_backward(const float* x, const float* v, int64_t m, int32_t n_freq, const float* gbar,
+                                             int64_t ldbar, const float* g_emb, int64_t ld, float* g_x, d3h_stream_t stream) {
+  const int e = 3 * (2 * n_freq + 1);
+  if (m < 0 || n_freq < 0 || n_freq > 16 || ld < e || (gbar && ldbar < e) || (m > 0 && (!x || !v || !g_emb || !g_x))) {
+    set_error("d3h_mlp_embed_second_backward: bad argument (g_emb, and gbar if given, hold the 3 (2 n_freq + 1) channels)");
+    return D3H_E_BADARG;
+  }
+  if (m == 0) return D3H_OK;
+  embed_second_backward_kernel<<<(unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, v, m, n_freq, gbar, ldbar,
+                                                                                             g_emb, ld, g_x);
+  return finish_launch("d3h_mlp_embed_second_backward");
+}
+
+extern "C" int d3h_mlp_head_second_backward(const float* adot, int64_t ldad, const float* a, int64_t lda, const float* delta,
+                                            int64_t ldd, const float* zdot, int64_t ldzd, int64_t m, int32_t k,
+                                            const float* g, int32_t d_out, float* dw, float* mu, int64_t ldmu,
+                                            d3h_stream_t stream) {
+  if (m < 0 || k <= 0 || k > 256 || (k % 4) || d_out <= 0 || d_out > 8 || !dw || (m > 0 && !g) ||
+      !operand_ok(adot, ldad, m, k) || !operand_ok(a, lda, m, k) || !operand_ok(delta, ldd, m, k) ||
+      !operand_ok(zdot, ldzd, m, k) || !operand_ok(mu, ldmu, m, k)) {
+    set_error("d3h_mlp_head_second_backward: bad argument (K <= 256 and a multiple of 4, 1 <= d_out <= 8, leading "
+              "dimensions multiples of 4, 16-byte aligned adot / a / delta / zdot / mu)");
+    return D3H_E_BADARG;
+  }
+  if (m == 0) return D3H_OK;
+  const unsigned blocks = (unsigned)((m + kHeadRows - 1) / kHeadRows);
+  cudaStream_t st = (cudaStream_t)stream;
+#define D3H_HEAD2(D) head_second_backward_kernel<D><<<blocks, 256, 0, st>>>(adot, ldad, a, lda, delta, ldd, zdot, ldzd, m, k, g, dw, mu, ldmu)
+  switch (d_out) {
+    case 1: D3H_HEAD2(1); break;
+    case 2: D3H_HEAD2(2); break;
+    case 3: D3H_HEAD2(3); break;
+    case 4: D3H_HEAD2(4); break;
+    case 5: D3H_HEAD2(5); break;
+    case 6: D3H_HEAD2(6); break;
+    case 7: D3H_HEAD2(7); break;
+    default: D3H_HEAD2(8); break;
+  }
+#undef D3H_HEAD2
+  return finish_launch("d3h_mlp_head_second_backward");
 }
 
 // point ranges of a wgrad call: two CTAs per SM and column tile, at least 16 slices (512 points) each

@@ -1,5 +1,7 @@
 """`Embedding`: drop-in for the reference module of the same name (geometry/embedding.py:4-38): x -> (x, sin(2^k x),
-cos(2^k x), ...), k < N_freqs.  The arithmetic runs in libd3h_tets.so (d3h_mlp_embed); CUDA tensors only."""
+cos(2^k x), ...), k < N_freqs.  The arithmetic runs in libd3h_tets.so (d3h_mlp_embed); CUDA tensors only.  Twice
+differentiable with respect to the points: under create_graph=True the backward pass is itself a Function whose gradient
+runs in d3h_mlp_embed_second_backward / d3h_mlp_embed_tangent (a third derivative raises NotImplementedError)."""
 from __future__ import annotations
 
 import torch
@@ -24,13 +26,53 @@ class _EmbedFn(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g):
         (x,) = ctx.saved_tensors
+        if torch.is_grad_enabled():          # create_graph=True: the adjoint as a differentiable Function of (x, g)
+            return _EmbedGradFn.apply(x, g, ctx.n_freq), None
+        return _embed_backward(x, g.contiguous().float(), ctx.n_freq), None
+
+
+def _embed_backward(x, g, n_freq):
+    gx = torch.empty_like(x)
+    with torch.cuda.device(x.device):
+        _cabi.check(_cabi.lib().d3h_mlp_embed_backward(x.data_ptr(), x.shape[0], n_freq, g.data_ptr(), g.shape[1],
+                                                       gx.data_ptr(), 0, torch.cuda.current_stream(x.device).cuda_stream),
+                    "d3h_mlp_embed_backward")
+    return gx
+
+
+class _EmbedGradFn(torch.autograd.Function):
+    """gx = E'(x)^T g, differentiable once: d/dx sum(v gx) = E''(x)[v]^T g (d3h_mlp_embed_second_backward), d/dg = E'(x) v
+    (d3h_mlp_embed_tangent).  A third derivative raises NotImplementedError."""
+
+    @staticmethod
+    def forward(ctx, x, g, n_freq):
         g = g.contiguous().float()
-        gx = torch.empty_like(x)
+        ctx.save_for_backward(x, g)
+        ctx.n_freq = n_freq
+        ctx.set_materialize_grads(False)
+        return _embed_backward(x, g, n_freq)
+
+    @staticmethod
+    def backward(ctx, v):
+        if torch.is_grad_enabled():
+            raise NotImplementedError("d3human-code_b200 Embedding: no third derivative (create_graph=True through the second one)")
+        if v is None:
+            return None, None, None
+        x, g = ctx.saved_tensors
+        v = v.contiguous().float()
+        m, c = x.shape[0], g.shape[1]
+        L = _cabi.lib()
         with torch.cuda.device(x.device):
-            _cabi.check(_cabi.lib().d3h_mlp_embed_backward(x.data_ptr(), x.shape[0], ctx.n_freq, g.data_ptr(), g.shape[1],
-                                                           gx.data_ptr(), 0, torch.cuda.current_stream(x.device).cuda_stream),
-                        "d3h_mlp_embed_backward")
-        return gx, None
+            st = torch.cuda.current_stream(x.device).cuda_stream
+            hx = torch.empty_like(x)
+            _cabi.check(L.d3h_mlp_embed_second_backward(x.data_ptr(), v.data_ptr(), m, ctx.n_freq, None, 0, g.data_ptr(), c,
+                                                        hx.data_ptr(), st), "d3h_mlp_embed_second_backward")
+            hg = None
+            if ctx.needs_input_grad[1]:
+                hg = torch.empty((m, c), dtype=torch.float32, device=x.device)
+                _cabi.check(L.d3h_mlp_embed_tangent(x.data_ptr(), v.data_ptr(), m, ctx.n_freq, hg.data_ptr(), c, c, st),
+                            "d3h_mlp_embed_tangent")
+        return hx, hg, None
 
 
 class Embedding(nn.Module):

@@ -9,8 +9,9 @@
  * iteration, and GEMM-shaped, so unlike the extraction it belongs on the tensor cores.
  *
  * The entry points below are the building blocks the Python host (d3human-code_b200/geometry/mlp.py, a drop-in for the
- * reference's `MLP` module with the same parameters / state_dict) chains for the forward and backward pass.  The GEMMs
- * run on the 5th-generation tensor cores (tcgen05.mma kind::tf32, accumulators in tensor memory) with the 3xTF32 split
+ * reference's `MLP` module with the same parameters / state_dict) chains for the forward and backward pass, and for the
+ * second derivative the eikonal term needs (section "Second derivative" below).  The GEMMs run on the 5th-generation
+ * tensor cores (tcgen05.mma kind::tf32, accumulators in tensor memory) with the 3xTF32 split
  *     a = a_hi + a_lo,  a_hi = a with the low 13 mantissa bits cleared:   a.b ~= a_hi.b_hi + a_lo.b_hi + a_hi.b_lo
  * so the results carry fp32-level error (~1e-6 relative, like a reordered fp32 sum) -- the reference computes in fp32
  * with TF32 disabled (torch default), and sign(sdf) decides the topology downstream.
@@ -82,6 +83,47 @@ int d3h_mlp_head(const float* a, int64_t lda, int64_t m, int32_t k, const float*
  * K <= 256 and a multiple of 4, lda / ldz multiples of 4, a / dz / w 16-byte aligned. */
 int d3h_mlp_head_backward(const float* a, int64_t lda, int64_t m, int32_t k, const float* w, int32_t d_out,
                           const float* g, float* dz, int64_t ldz, float* dw, float* db, d3h_stream_t stream);
+
+/* ---- Second derivative (the eikonal term: autograd.grad(sdf, x, create_graph=True), then a loss on that gradient).
+ * With delta_l the gradient at the pre-activation z_l of hidden layer l from the first backward pass, g_emb the gradient at
+ * the encoding, and an upstream v (M, 3) for the first backward's g_x: a tangent pass along x' = v (e' = E'(x) v,
+ * z'_l = h'_l W_l^T, a'_l = z'_l * softplus'(z_l)), then an adjoint pass from the output layer down
+ *     mu_l      = (mu_{l+1} W_{l+1})[activation part] * softplus'(z_l) + beta [beta a_l <= 20] exp(-beta a_l) delta_l z'_l
+ *     dW_l     += mu_l^T h_l + delta_l^T h'_l,  db_l += sum mu_l     (d3h_mlp_wgrad, two calls per input block)
+ *     gbar     += (mu_l W_l)[encoding part]
+ *     g_x       = E'(x)^T gbar + E''(x)[v]^T g_emb
+ * with softplus'' recovered from the saved output a = softplus(z) as in mode 2 of d3h_mlp_linear and zero past the
+ * threshold, as torch's softplus double backward. */
+
+/* e' = E'(x) v: out[m, 0:3] = v[m], out[m, 3+6k+d] = 2^k cos(2^k x) v, out[m, 6+6k+d] = -2^k sin(2^k x) v; columns up to
+ * n_cols are zeroed.  Layout rules as d3h_mlp_embed (x, v (M, 3) contiguous). */
+int d3h_mlp_embed_tangent(const float* x, const float* v, int64_t m, int32_t n_freq, float* out, int64_t ld, int32_t n_cols,
+                          d3h_stream_t stream);
+
+/* g_x[m] = E'(x)^T gbar[m] + sum_k -4^k v (sin(2^k x) g_emb_sin_k + cos(2^k x) g_emb_cos_k), overwritten.  gbar may be NULL
+ * (the standalone Embedding: only the second term). */
+int d3h_mlp_embed_second_backward(const float* x, const float* v, int64_t m, int32_t n_freq, const float* gbar,
+                                  int64_t ldbar, const float* g_emb, int64_t ld, float* g_x, d3h_stream_t stream);
+
+/* Tangent through one hidden layer, same GEMM as d3h_mlp_linear (no bias): zdot = a B^T, adot = zdot * softplus'(z) with
+ * softplus' from the layer's saved output y (M, ldy).  Rules of d3h_mlp_linear; y / zdot / adot hold N columns. */
+int d3h_mlp_linear_tangent(const float* a, int64_t lda, int64_t m, int32_t k, const float* w_packed, int32_t n,
+                           const float* y, int64_t ldy, float* zdot, int64_t ldzd, float* adot, int64_t ldad,
+                           d3h_stream_t stream);
+
+/* Adjoint step: c = (a B^T) * softplus'(z) + beta [beta y <= 20] exp(-beta y) * delta * zdot, where y, delta and zdot are
+ * the saved output, first-backward gradient and tangent of the layer that produced the GEMM's output columns.  Rules of
+ * d3h_mlp_linear; y / delta / zdot / c hold N columns. */
+int d3h_mlp_linear_adjoint(const float* a, int64_t lda, int64_t m, int32_t k, const float* w_packed, int32_t n,
+                           const float* y, int64_t ldy, const float* delta, int64_t ldd, const float* zdot, int64_t ldzd,
+                           float* c, int64_t ldc, d3h_stream_t stream);
+
+/* The output layer's share in one sweep: dw[j, k] += sum_m g[m, j] adot[m, k] (ACCUMULATE; the output bias gets no second
+ * derivative) and mu[m, k] = beta [beta a <= 20] exp(-beta a) delta zdot for the last hidden layer (a, delta, zdot at m, k).
+ * K <= 256 and a multiple of 4, leading dimensions multiples of 4, adot / a / delta / zdot / mu 16-byte aligned. */
+int d3h_mlp_head_second_backward(const float* adot, int64_t ldad, const float* a, int64_t lda, const float* delta,
+                                 int64_t ldd, const float* zdot, int64_t ldzd, int64_t m, int32_t k, const float* g,
+                                 int32_t d_out, float* dw, float* mu, int64_t ldmu, d3h_stream_t stream);
 
 #ifdef __cplusplus
 }
