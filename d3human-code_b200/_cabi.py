@@ -154,8 +154,8 @@ def lib() -> C.CDLL:
     L.d3h_mesh_normals_backward.restype = C.c_int
     L.d3h_mesh_normals_backward.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                             C.c_void_p]
-    # include/d3h_mlp.h (the CPU emulation of tests/emu has no tensor-core stage: its library lacks these symbols; the
-    # real library always exports them, tests/test_cabi.py)
+    # include/d3h_mlp.h (both the real library and the CPU emulation of tests/emu export them, tests/test_cabi.py and
+    # tests/test_emu_parity.py)
     if hasattr(L, "d3h_mlp_linear"):
         vp, i64, i32 = C.c_void_p, C.c_int64, C.c_int32
         L.d3h_mlp_embed.restype = C.c_int

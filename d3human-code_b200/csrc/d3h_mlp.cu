@@ -25,8 +25,9 @@
 //                     and a on their way into shared memory (lanes <-> points, conflict-free), every CTA owns a point
 //                     range and 128 of dz's columns and adds its partial result to dw with red.global.add.f32.
 //
-// No CPU emulation of this file (tests/emu does not list it): tensor-core instructions have no stand-in there; the
-// parity tests of this stage are GPU-only and compare against oracle/mlp_oracle.py (float64).
+// The CPU emulation of tests/emu builds this file too: its D3H_CPU_EMU branches of the PTX wrappers call the emulator's
+// mbarriers, bulk copies, tensor memory and tcgen05 instructions (modelled from the PTX ISA, not from these helpers), and
+// tests/test_emu_mlp.py runs the edge cases of tests/test_zzzzzzzzz_mlp_edges.py against oracle/mlp_oracle.py (float64).
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -46,6 +47,7 @@ constexpr float kBeta = 100.f, kThreshold = 20.f;     // nn.Softplus(beta=100), 
 // ---------------------------------------------------------------------------------------------- PTX wrappers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
+#ifndef D3H_CPU_EMU
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
 }
@@ -123,6 +125,44 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
 #pragma unroll
   for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
 }
+// the dynamic shared memory of a kernel, and kernel<<<grid, block, smem, stream>>>
+#define D3H_DYN_SMEM(name) extern __shared__ __align__(1024) uint8_t name[]
+#define D3H_LAUNCH(kernel, grid, block, smem, stream) kernel<<<grid, block, smem, stream>>>
+#else
+// tests/emu (functional CPU emulation of the kernels, test infrastructure only): no PTX -- the emulator's mbarriers,
+// bulk copies, tensor memory and tcgen05 instructions (tests/emu/emu_core.cpp), no <<< >>>
+__device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) { emu::mbar_init(bar, count); }
+__device__ __forceinline__ void mbar_arrive(uint64_t* bar) { emu::mbar_arrive(bar); }
+__device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) { emu::mbar_wait(bar, parity); }
+__device__ __forceinline__ void fence_proxy_async() {}
+__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) { emu::mbar_arrive_expect_tx(bar, bytes); }
+__device__ __forceinline__ void bulk_copy_g2s(void* dst_smem, const void* src, uint32_t bytes, uint64_t* bar) {
+  emu::bulk_copy_g2s(dst_smem, src, bytes, bar);
+}
+__device__ __forceinline__ void fence_barrier_init() {}
+__device__ __forceinline__ void tc_fence_before() {}
+__device__ __forceinline__ void tc_fence_after() {}
+__device__ __forceinline__ void tmem_alloc(uint32_t* dst_smem, uint32_t cols) {   // whole warp
+  if ((threadIdx.x & 31u) == 0) emu::tmem_alloc(dst_smem, cols);
+  __syncwarp();
+}
+__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {     // whole warp
+  __syncwarp();
+  if ((threadIdx.x & 31u) == 0) emu::tmem_dealloc(taddr, cols);
+}
+__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc,
+                                          uint32_t accumulate) {
+  emu::mma_tf32(tmem_d, desc_a, desc_b, idesc, accumulate);
+}
+__device__ __forceinline__ void umma_commit(uint64_t* bar) { emu::mma_commit(bar); }
+__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
+  uint32_t r[32];
+  emu::tmem_ld_32x32b_x32(taddr, r);
+  for (int i = 0; i < 32; ++i) v[i] = __uint_as_float(r[i]);
+}
+#define D3H_DYN_SMEM(name) uint8_t* const name = emu::dyn_smem()
+#define D3H_LAUNCH(kernel, grid, block, smem, stream) emu_launch(kernel, grid, block, smem, stream)
+#endif
 
 // Shared-memory matrix descriptor of a K-major SWIZZLE_128B tile (rows of 128 bytes, 8-row atoms 1024 bytes apart):
 // start address and offsets in 16-byte units; leading byte offset 1 (unused with swizzle), stride byte offset 64,
@@ -244,7 +284,7 @@ constexpr int kEpiFirstOrder = 0, kEpiTangent = 1, kEpiAdjoint = 2;
 // ---------------------------------------------------------------------------------------------- c = f(a w^T + bias)
 template <int kEpi>
 __global__ void __launch_bounds__(kThreads, kCtasPerSm) mlp_linear_kernel(LinearArgs g) {
-  extern __shared__ __align__(1024) uint8_t smem[];
+  D3H_DYN_SMEM(smem);
   __shared__ uint64_t s_full, s_empty, s_done;
   __shared__ uint32_t s_tmem;
   const StageBuffers sl = stage_layout(g.n);
@@ -395,7 +435,7 @@ struct WgradArgs {
 // (the k index of the MMA), warp w takes the 16-byte column groups w, w + 8, ... of that point's row, and the four values
 // of a group go to four tile rows at k = lane (32 lanes -> 32 distinct words of one 128-byte row: no bank conflict).
 __global__ void __launch_bounds__(kThreads, kCtasPerSm) mlp_wgrad_kernel(WgradArgs g) {
-  extern __shared__ __align__(1024) uint8_t smem[];
+  D3H_DYN_SMEM(smem);
   __shared__ uint64_t s_full, s_empty, s_done;
   __shared__ uint32_t s_tmem;
   const StageBuffers sl = stage_layout(g.k);
@@ -795,7 +835,7 @@ static void launch_linear(const LinearArgs& g, d3h_stream_t stream) {
     cudaFuncSetAttribute(mlp_linear_kernel<kEpi>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)stage_layout(256).bytes);
     attr = true;
   }
-  mlp_linear_kernel<kEpi><<<(unsigned)((g.m + kTileM - 1) / kTileM), kThreads, stage_layout(g.n).bytes, (cudaStream_t)stream>>>(g);
+  D3H_LAUNCH(mlp_linear_kernel<kEpi>, (unsigned)((g.m + kTileM - 1) / kTileM), kThreads, stage_layout(g.n).bytes, (cudaStream_t)stream)(g);
 }
 
 extern "C" int d3h_mlp_embed(const float* x, int64_t m, int32_t n_freq, float* out, int64_t ld, int32_t n_cols,
@@ -806,9 +846,9 @@ extern "C" int d3h_mlp_embed(const float* x, int64_t m, int32_t n_freq, float* o
   }
   if (m == 0) return D3H_OK;
   if ((n_cols % 4) == 0 && (ld % 4) == 0 && aligned16(out))
-    embed4_kernel<<<(unsigned)((m * (n_cols / 4) + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, m, n_freq, out, ld, n_cols);
+    D3H_LAUNCH(embed4_kernel, (unsigned)((m * (n_cols / 4) + 255) / 256), 256, 0, (cudaStream_t)stream)(x, m, n_freq, out, ld, n_cols);
   else
-    embed_kernel<<<(unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, m, n_freq, out, ld, n_cols);
+    D3H_LAUNCH(embed_kernel, (unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream)(x, m, n_freq, out, ld, n_cols);
   return finish_launch("d3h_mlp_embed");
 }
 
@@ -819,7 +859,7 @@ extern "C" int d3h_mlp_embed_backward(const float* x, int64_t m, int32_t n_freq,
     return D3H_E_BADARG;
   }
   if (m == 0) return D3H_OK;
-  embed_backward_kernel<<<(unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, m, n_freq, g_emb, ld, g_x, accumulate);
+  D3H_LAUNCH(embed_backward_kernel, (unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream)(x, m, n_freq, g_emb, ld, g_x, accumulate);
   return finish_launch("d3h_mlp_embed_backward");
 }
 
@@ -836,7 +876,7 @@ extern "C" int d3h_mlp_pack_weight(const float* w, int64_t ldw, int32_t n_valid,
   }
   PackArgs g{w, ldw, packed, n_valid, k_valid, transpose ? 1 : 0, row0, col0, n_pad, k_pad};
   const int64_t total = (int64_t)n_pad * (k_pad / 4);
-  mlp_pack_weight_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(g);
+  D3H_LAUNCH(mlp_pack_weight_kernel, (unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream)(g);
   return finish_launch("d3h_mlp_pack_weight");
 }
 
@@ -903,7 +943,7 @@ extern "C" int d3h_mlp_embed_tangent(const float* x, const float* v, int64_t m, 
     return D3H_E_BADARG;
   }
   if (m == 0) return D3H_OK;
-  embed_tangent_kernel<<<(unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, v, m, n_freq, out, ld, n_cols);
+  D3H_LAUNCH(embed_tangent_kernel, (unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream)(x, v, m, n_freq, out, ld, n_cols);
   return finish_launch("d3h_mlp_embed_tangent");
 }
 
@@ -915,7 +955,7 @@ extern "C" int d3h_mlp_embed_second_backward(const float* x, const float* v, int
     return D3H_E_BADARG;
   }
   if (m == 0) return D3H_OK;
-  embed_second_backward_kernel<<<(unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, v, m, n_freq, gbar, ldbar,
+  D3H_LAUNCH(embed_second_backward_kernel, (unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream)(x, v, m, n_freq, gbar, ldbar,
                                                                                              g_emb, ld, g_x);
   return finish_launch("d3h_mlp_embed_second_backward");
 }
@@ -934,7 +974,7 @@ extern "C" int d3h_mlp_head_second_backward(const float* adot, int64_t ldad, con
   if (m == 0) return D3H_OK;
   const unsigned blocks = (unsigned)((m + kHeadRows - 1) / kHeadRows);
   cudaStream_t st = (cudaStream_t)stream;
-#define D3H_HEAD2(D) head_second_backward_kernel<D><<<blocks, 256, 0, st>>>(adot, ldad, a, lda, delta, ldd, zdot, ldzd, m, k, g, dw, mu, ldmu)
+#define D3H_HEAD2(D) D3H_LAUNCH(head_second_backward_kernel<D>, blocks, 256, 0, st)(adot, ldad, a, lda, delta, ldd, zdot, ldzd, m, k, g, dw, mu, ldmu)
   switch (d_out) {
     case 1: D3H_HEAD2(1); break;
     case 2: D3H_HEAD2(2); break;
@@ -991,9 +1031,9 @@ extern "C" int d3h_mlp_wgrad(const float* dz, int64_t ldz, const float* a, int64
   float* part = reinterpret_cast<float*>(workspace);
   float* part_b = db ? part + ranges * (int64_t)n * k : nullptr;
   WgradArgs g{dz, ldz, a, lda, part, part_b, m, per, n, k};
-  mlp_wgrad_kernel<<<dim3((unsigned)ranges, (unsigned)(n / kTileM)), kThreads, smem, (cudaStream_t)stream>>>(g);
+  D3H_LAUNCH(mlp_wgrad_kernel, dim3((unsigned)ranges, (unsigned)(n / kTileM)), kThreads, smem, (cudaStream_t)stream)(g);
   const int64_t total = (int64_t)n * k + (db ? n : 0);
-  wgrad_reduce_kernel<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(part, part_b, (int)ranges, n, k, dw, lddw, db);
+  D3H_LAUNCH(wgrad_reduce_kernel, (unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream)(part, part_b, (int)ranges, n, k, dw, lddw, db);
   return finish_launch("d3h_mlp_wgrad");
 }
 
@@ -1004,7 +1044,7 @@ extern "C" int d3h_mlp_head(const float* a, int64_t lda, int64_t m, int32_t k, c
     return D3H_E_BADARG;
   }
   if (m == 0) return D3H_OK;
-  head_kernel<<<(unsigned)((m + 7) / 8), 256, 0, (cudaStream_t)stream>>>(a, lda, m, k, w, bias, d_out, out);
+  D3H_LAUNCH(head_kernel, (unsigned)((m + 7) / 8), 256, 0, (cudaStream_t)stream)(a, lda, m, k, w, bias, d_out, out);
   return finish_launch("d3h_mlp_head");
 }
 
@@ -1020,14 +1060,14 @@ extern "C" int d3h_mlp_head_backward(const float* a, int64_t lda, int64_t m, int
   const unsigned blocks = (unsigned)((m + kHeadRows - 1) / kHeadRows);
   cudaStream_t st = (cudaStream_t)stream;
   switch (d_out) {
-    case 1: head_backward_kernel<1><<<blocks, 256, 0, st>>>(a, lda, m, k, w, g, dz, ldz, dw, db); break;
-    case 2: head_backward_kernel<2><<<blocks, 256, 0, st>>>(a, lda, m, k, w, g, dz, ldz, dw, db); break;
-    case 3: head_backward_kernel<3><<<blocks, 256, 0, st>>>(a, lda, m, k, w, g, dz, ldz, dw, db); break;
-    case 4: head_backward_kernel<4><<<blocks, 256, 0, st>>>(a, lda, m, k, w, g, dz, ldz, dw, db); break;
-    case 5: head_backward_kernel<5><<<blocks, 256, 0, st>>>(a, lda, m, k, w, g, dz, ldz, dw, db); break;
-    case 6: head_backward_kernel<6><<<blocks, 256, 0, st>>>(a, lda, m, k, w, g, dz, ldz, dw, db); break;
-    case 7: head_backward_kernel<7><<<blocks, 256, 0, st>>>(a, lda, m, k, w, g, dz, ldz, dw, db); break;
-    default: head_backward_kernel<8><<<blocks, 256, 0, st>>>(a, lda, m, k, w, g, dz, ldz, dw, db); break;
+    case 1: D3H_LAUNCH(head_backward_kernel<1>, blocks, 256, 0, st)(a, lda, m, k, w, g, dz, ldz, dw, db); break;
+    case 2: D3H_LAUNCH(head_backward_kernel<2>, blocks, 256, 0, st)(a, lda, m, k, w, g, dz, ldz, dw, db); break;
+    case 3: D3H_LAUNCH(head_backward_kernel<3>, blocks, 256, 0, st)(a, lda, m, k, w, g, dz, ldz, dw, db); break;
+    case 4: D3H_LAUNCH(head_backward_kernel<4>, blocks, 256, 0, st)(a, lda, m, k, w, g, dz, ldz, dw, db); break;
+    case 5: D3H_LAUNCH(head_backward_kernel<5>, blocks, 256, 0, st)(a, lda, m, k, w, g, dz, ldz, dw, db); break;
+    case 6: D3H_LAUNCH(head_backward_kernel<6>, blocks, 256, 0, st)(a, lda, m, k, w, g, dz, ldz, dw, db); break;
+    case 7: D3H_LAUNCH(head_backward_kernel<7>, blocks, 256, 0, st)(a, lda, m, k, w, g, dz, ldz, dw, db); break;
+    default: D3H_LAUNCH(head_backward_kernel<8>, blocks, 256, 0, st)(a, lda, m, k, w, g, dz, ldz, dw, db); break;
   }
   return finish_launch("d3h_mlp_head_backward");
 }

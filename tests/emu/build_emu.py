@@ -10,7 +10,7 @@ CSRC = os.path.join(ROOT, "d3human-code_b200", "csrc")
 OUT = os.path.join(HERE, "_build", "libd3h_tets_emu.so")
 OUT_SAN = os.path.join(HERE, "_build", "libd3h_tets_emu_san.so")
 OUT_TSAN = os.path.join(HERE, "_build", "libd3h_tets_emu_tsan.so")
-SOURCES = ["d3h_api.cu", "d3h_classify.cu", "d3h_sort.cu", "d3h_scan.cu", "d3h_surface.cu", "d3h_backward.cu", "d3h_mesh.cu", "d3h_lbs.cu"]
+SOURCES = ["d3h_api.cu", "d3h_classify.cu", "d3h_sort.cu", "d3h_scan.cu", "d3h_surface.cu", "d3h_backward.cu", "d3h_mesh.cu", "d3h_lbs.cu", "d3h_mlp.cu"]
 
 
 def build(force=False, sanitize=False, tsan=False):
@@ -19,7 +19,7 @@ def build(force=False, sanitize=False, tsan=False):
     misaligned vector loads / stores and out-of-range local array indices abort the run."""
     out = OUT_TSAN if tsan else (OUT_SAN if sanitize else OUT)
     deps = [os.path.join(CSRC, f) for f in os.listdir(CSRC)] + [os.path.join(HERE, f) for f in ("cuda_runtime.h", "emu_core.cpp")]
-    deps += [os.path.join(ROOT, "include", h) for h in ("d3h_tets.h", "d3h_mesh.h", "d3h_lbs.h")]
+    deps += [os.path.join(ROOT, "include", h) for h in ("d3h_tets.h", "d3h_mesh.h", "d3h_lbs.h", "d3h_mlp.h")]
     if not force and os.path.isfile(out) and all(os.path.getmtime(d) <= os.path.getmtime(out) for d in deps):
         return out
     os.makedirs(os.path.dirname(out), exist_ok=True)

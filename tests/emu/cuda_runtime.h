@@ -57,7 +57,7 @@ static inline float4 make_float4(float a, float b, float c, float d) { return {a
 namespace emu {
 struct Idx { unsigned x, y, z; };
 extern Idx g_threadIdx, g_blockIdx, g_blockDim, g_gridDim;
-void run_grid(dim3 grid, dim3 block, const std::function<void()>& body);
+void run_grid(dim3 grid, dim3 block, const std::function<void()>& body, size_t dyn_smem_bytes = 0);
 void block_barrier();
 // warp collective: every lane of `mask` contributes `v`; returns the contributions of all 32 lanes (undefined for lanes
 // outside the mask) through `out`
@@ -66,6 +66,27 @@ unsigned long long now_ns();
 void set_shuffle(unsigned long long seed);
 void warp_sync_release();
 void warp_sync_acquire();
+// dynamic shared memory of the running block (1024-byte aligned, poisoned with 0xCB before every block) and its size
+unsigned char* dyn_smem();
+size_t dyn_smem_bytes();
+size_t cvta_generic_to_shared(const void* p);
+// the asynchronous part of sm_100 that csrc/d3h_mlp.cu uses: mbarriers, bulk copies global -> shared, tensor memory and
+// tcgen05 (emu_core.cpp, written from the PTX ISA's definitions)
+void mbar_init(uint64_t* bar, unsigned count);
+void mbar_arrive(uint64_t* bar);
+void mbar_arrive_expect_tx(uint64_t* bar, unsigned bytes);
+void mbar_wait(uint64_t* bar, unsigned parity);
+void bulk_copy_g2s(void* dst, const void* src, unsigned bytes, uint64_t* bar);
+void tmem_alloc(uint32_t* dst, unsigned cols);
+void tmem_dealloc(uint32_t taddr, unsigned cols);
+void mma_tf32(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, unsigned accumulate);
+void mma_commit(uint64_t* bar);
+void tmem_ld_32x32b_x32(uint32_t taddr, uint32_t (&r)[32]);
+// launches: the runtime's error of the last launch, and the dynamic shared memory limit a kernel was given
+int take_last_error();
+void set_last_error(int e);
+int func_max_dynamic_smem(const void* f);
+void set_func_max_dynamic_smem(const void* f, int bytes);
 }  // namespace emu
 // the built-in variables are plain globals (references): struct members named gridDim / blockDim keep working
 static emu::Idx& threadIdx = emu::g_threadIdx;
@@ -169,6 +190,16 @@ static inline float __fmul_rn(float a, float b) { volatile float r = a * b; retu
 static inline float __fdiv_rn(float a, float b) { volatile float r = a / b; return r; }
 static inline float __fmaf_rn(float a, float b, float c) { return fmaf(a, b, c); }
 static inline float __fsqrt_rn(float a) { return sqrtf(a); }
+static inline float __uint_as_float(unsigned u) { float f; memcpy(&f, &u, 4); return f; }
+static inline unsigned __float_as_uint(float f) { unsigned u; memcpy(&u, &f, 4); return u; }
+// the fast intrinsics as the GPU evaluates them: __expf(x) = ex2.approx(x * log2(e)), __logf(x) = lg2.approx(x) * ln(2),
+// with the multiplications rounded to fp32 (ex2 / lg2 themselves are within 2 ulp; the libm functions stand in for them)
+// (glibc declares functions of these names itself: the intrinsics are macros)
+static inline float emu_expf(float x) { volatile float t = x * 1.44269504088896341f; return exp2f(t); }
+static inline float emu_logf(float x) { volatile float t = log2f(x); return t * 0.693147180559945309f; }
+#define __expf(x) emu_expf(x)
+#define __logf(x) emu_logf(x)
+static inline size_t __cvta_generic_to_shared(const void* p) { return emu::cvta_generic_to_shared(p); }
 template <typename T> static inline T __ldg(const T* p) { return *p; }
 template <typename T> static inline T emu_load_relaxed(const T* p);
 template <typename T> static inline T __ldcg(const T* p) { return emu_load_relaxed(p); }  // L2 loads: may watch atomics
@@ -274,7 +305,7 @@ static inline float4 atomicAdd(float4* p, float4 v) {  // the hardware's vector 
 
 // ---- runtime API: one device, memory = host memory, streams / events are no-ops, graphs unsupported -------------------
 typedef int cudaError_t;
-enum { cudaSuccess = 0, cudaErrorNotSupported = 801 };
+enum { cudaSuccess = 0, cudaErrorInvalidValue = 1, cudaErrorNotSupported = 801 };
 typedef struct emu_stream_s* cudaStream_t;
 typedef struct emu_event_s* cudaEvent_t;
 typedef struct emu_graph_s* cudaGraph_t;
@@ -296,14 +327,19 @@ struct cudaLaunchAttributeValue { int priority; };
 struct cudaLaunchAttribute { cudaLaunchAttributeID id; cudaLaunchAttributeValue val; };
 struct cudaLaunchConfig_t { dim3 gridDim, blockDim; size_t dynamicSmemBytes; cudaStream_t stream; cudaLaunchAttribute* attrs; unsigned numAttrs; };
 
-static inline const char* cudaGetErrorString(cudaError_t e) { return e == 0 ? "no error" : "emulation: unsupported"; }
-static inline cudaError_t cudaGetLastError() { return cudaSuccess; }
+static inline const char* cudaGetErrorString(cudaError_t e) {
+  return e == 0 ? "no error" : (e == cudaErrorInvalidValue ? "invalid argument" : "emulation: unsupported");
+}
+static inline cudaError_t cudaGetLastError() { return emu::take_last_error(); }
 static inline cudaError_t cudaGetDevice(int* d) { *d = 0; return cudaSuccess; }
 static inline cudaError_t cudaDeviceGetAttribute(int* v, cudaDeviceAttr, int) { *v = 4; return cudaSuccess; }
 static inline cudaError_t cudaDeviceSynchronize() { return cudaSuccess; }
 static inline cudaError_t cudaDeviceGetStreamPriorityRange(int* lo, int* hi) { *lo = 0; *hi = -5; return cudaSuccess; }
 static inline cudaError_t cudaOccupancyMaxActiveBlocksPerMultiprocessor(int* n, const void*, int, size_t) { *n = 2; return cudaSuccess; }
-template <typename F> static inline cudaError_t cudaFuncSetAttribute(F, cudaFuncAttribute, int) { return cudaSuccess; }
+template <typename F> static inline cudaError_t cudaFuncSetAttribute(F f, cudaFuncAttribute a, int v) {
+  if (a == cudaFuncAttributeMaxDynamicSharedMemorySize) emu::set_func_max_dynamic_smem(reinterpret_cast<const void*>(f), v);
+  return cudaSuccess;
+}
 static inline cudaError_t cudaStreamCreateWithFlags(cudaStream_t* s, unsigned) { *s = nullptr; return cudaSuccess; }
 static inline cudaError_t cudaStreamCreateWithPriority(cudaStream_t* s, unsigned, int) { *s = nullptr; return cudaSuccess; }
 static inline cudaError_t cudaStreamWaitEvent(cudaStream_t, cudaEvent_t, unsigned) { return cudaSuccess; }
@@ -338,7 +374,33 @@ static inline cudaError_t cudaFree(void* p) { free(p); return cudaSuccess; }
 
 template <typename... KArgs, typename... Args>
 static inline cudaError_t cudaLaunchKernelEx(const cudaLaunchConfig_t* cfg, void (*kernel)(KArgs...), Args&&... args) {
+  // more than 48 KB of dynamic shared memory needs the kernel's cudaFuncAttributeMaxDynamicSharedMemorySize first: the
+  // launch fails with cudaErrorInvalidValue (reported by the next cudaGetLastError) and nothing runs
+  if (cfg->dynamicSmemBytes > 48u * 1024u &&
+      (int64_t)cfg->dynamicSmemBytes > (int64_t)emu::func_max_dynamic_smem(reinterpret_cast<const void*>(kernel))) {
+    emu::set_last_error(cudaErrorInvalidValue);
+    return cudaErrorInvalidValue;
+  }
   auto body = [=]() { kernel(args...); };
-  emu::run_grid(cfg->gridDim, cfg->blockDim, body);
+  emu::run_grid(cfg->gridDim, cfg->blockDim, body, cfg->dynamicSmemBytes);
   return cudaSuccess;
+}
+// kernel<<<grid, block, smem, stream>>>(args) of the product sources, spelled EMU_LAUNCH(kernel, grid, block, smem, stream)(args)
+template <typename... KArgs>
+struct EmuLaunch {
+  void (*kernel)(KArgs...);
+  cudaLaunchConfig_t cfg;
+  template <typename... Args>
+  void operator()(Args&&... args) const { cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...); }
+};
+template <typename... KArgs>
+static inline EmuLaunch<KArgs...> emu_launch(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream) {
+  EmuLaunch<KArgs...> l;
+  memset(&l.cfg, 0, sizeof(l.cfg));
+  l.kernel = kernel;
+  l.cfg.gridDim = grid;
+  l.cfg.blockDim = block;
+  l.cfg.dynamicSmemBytes = smem;
+  l.cfg.stream = stream;
+  return l;
 }

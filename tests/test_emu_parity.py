@@ -115,8 +115,6 @@ def test_emulated_library_is_the_real_abi(dev):
     L = _cabi.lib()
     assert L.d3h_version() == _cabi.VERSION
     for name in _cabi.EXPORTED_SYMBOLS:
-        if name.startswith(("d3h_mlp_", "d3h_lbs_")):      # csrc/d3h_mlp.cu (tensor cores) and d3h_lbs.cu are GPU-tested only
-            continue
         assert hasattr(L, name)
 
 

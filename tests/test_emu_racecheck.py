@@ -19,6 +19,7 @@ SELECTION = [                              # ~40 s: every golden case on the thr
     "tests/test_emu_parity.py::test_tangent_gradients",
     "tests/test_emu_parity.py::test_fused_frames_shared_topology_and_regrowth",   # fused frames, shared / kept topology
     "tests/test_emu_lbs.py",                                                      # the skinning kernels at their edges (+30 s)
+    "tests/test_emu_mlp.py",                                                      # the SDF network: mbarrier pipeline, tcgen05
 ]
 FULL = SELECTION + [                       # D3H_RACECHECK_FULL=1: another four minutes (clean at the end of round 2)
     "tests/test_emu_mesh.py",

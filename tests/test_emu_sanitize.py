@@ -21,6 +21,7 @@ SELECTION = [                             # ~40 s: every golden case on the thre
     "tests/test_emu_parity.py::test_fused_frames_shared_topology_and_regrowth",   # fused frames, shared / kept topology
     "tests/test_emu_parity.py::test_compact_gradient_return",
     "tests/test_emu_lbs.py",                                                      # the skinning kernels at their edges (+50 s)
+    "tests/test_emu_mlp.py",                                                      # the SDF network at its edges
 ]
 FULL = SELECTION + [                      # D3H_SAN_FULL=1: another four minutes (clean at the end of round 2)
     "tests/test_emu_mesh.py",

@@ -5,12 +5,14 @@ writer, a counter consumed before every block has added to it, or a test that ex
 fails under some seed.  The second seed also POISONS every `torch.empty` / `torch.empty_like` result (0xCB bytes): on the
 GPU fresh allocations and reused workspaces hold arbitrary data, so nothing may rely on zero-filled scratch or outputs.
 A selection of the emulated parity tests, two seeds each.  Test infrastructure only."""
+import contextlib
 import ctypes
 
 import pytest
 import torch
 
 from tests import test_emu_mesh as EM
+from tests import test_emu_mlp as EMLP
 from tests import test_emu_parity as EP
 from tests import test_zz_mesh as ZM
 
@@ -79,3 +81,30 @@ def test_mesh_soups(shuffled, mesh_dev):
         ZM.test_random_triangle_soups(mesh_dev, seed)
     for seed in (0, 5, 15):
         ZM.test_degenerate_soups(mesh_dev, seed)
+
+
+mlp_dev = EMLP.dev                      # SDF network: the C ABI of the emulated library with CPU buffers
+
+
+@pytest.fixture
+def mlp_module_dev(mlp_dev, monkeypatch):
+    """geometry/mlp.py on CPU tensors that pass as CUDA tensors (as test_emu_mlp.module_dev)"""
+    monkeypatch.setattr(torch.Tensor, "is_cuda", property(lambda self: True))
+    monkeypatch.setattr(torch.cuda, "current_stream", lambda dev=None: EP._Stream())
+    monkeypatch.setattr(torch.cuda, "device", lambda dev=None: contextlib.nullcontext())
+    return mlp_dev
+
+
+@pytest.mark.parametrize("m,n,k", [(129, 192, 96), (257, 256, 288)])
+def test_mlp_linear(shuffled, mlp_dev, m, n, k):
+    for epi in ("mode1", "adjoint"):
+        EMLP.T.linear_case(mlp_dev, m, n, k, epi)
+
+
+def test_mlp_wgrad_and_head(shuffled, mlp_dev):
+    EMLP.T.wgrad_case(mlp_dev, 2000, 128, 192, True)
+    EMLP.T.head_case(mlp_dev, 3, 252, 513)
+
+
+def test_mlp_module(shuffled, mlp_module_dev):
+    EMLP.T.module_case(mlp_module_dev, "f11_d256_o8_skip_last", 129, True)

@@ -1,6 +1,6 @@
 """SDF field query on the tensor cores (SURVEY 8f row 3; include/d3h_mlp.h, d3human-code_b200/geometry/mlp.py) against
 the float64 oracle (oracle/mlp_oracle.py) and the golden vectors written from the live reference module
-(tests/golden/mlp_*.npz).  GPU only: tcgen05 has no CPU emulation.  Last file of the suite: a new stage must not stop
+(tests/golden/mlp_*.npz).  GPU only (the edge cases of tests/test_zzzzzzzzz_mlp_edges.py also run on the CPU emulation).  Last file of the suite: a new stage must not stop
 (-x) the tests of the extraction.
 
 Tolerances.  The reference computes in fp32 (TF32 off, torch default); the kernels use the 3xTF32 split with fp32
