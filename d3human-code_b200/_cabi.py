@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "lib", "libd3h_tets.so")
 
 D3H_OK, D3H_E_BADARG, D3H_E_CUDA, D3H_E_SMALLWS, D3H_E_TIMEOUT = 0, -1, -2, -3, -4
-VERSION = 500
+VERSION = 501
 
 #: every symbol include/d3h_tets.h declares (tests/test_cabi.py checks the library exports all of them)
 EXPORTED_SYMBOLS = (
@@ -20,6 +20,7 @@ EXPORTED_SYMBOLS = (
     "d3h_backward_workspace_bytes",
     "d3h_pack_tets_i64", "d3h_check_tets_i32", "d3h_extract_forward", "d3h_wait_counts", "d3h_extract_backward",
     "d3h_extract_forward_batch", "d3h_extract_forward_batch_nojoin", "d3h_lanes_join", "d3h_extract_backward_batch", "d3h_tangent_backward", "d3h_gather_rows", "d3h_classify_range", "d3h_extract_from_records",
+    "d3h_sdf_reg_workspace_bytes", "d3h_sdf_reg_forward", "d3h_sdf_reg_backward",
     "d3h_mesh_edges_workspace_bytes", "d3h_mesh_edges", "d3h_mesh_wait_counts", "d3h_mesh_normals_forward",
     "d3h_mesh_normals_backward",
     "d3h_lbs_blend", "d3h_lbs_blend_backward", "d3h_lbs_nearest_workspace_bytes", "d3h_lbs_nearest", "d3h_lbs_apply",
@@ -140,6 +141,14 @@ def lib() -> C.CDLL:
     L.d3h_classify_range.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
     L.d3h_extract_from_records.restype = C.c_int
     L.d3h_extract_from_records.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.c_int64, C.c_void_p]
+    L.d3h_sdf_reg_workspace_bytes.restype = C.c_int64
+    L.d3h_sdf_reg_workspace_bytes.argtypes = [C.c_int64, C.c_int64]
+    L.d3h_sdf_reg_forward.restype = C.c_int
+    L.d3h_sdf_reg_forward.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
+    L.d3h_sdf_reg_backward.restype = C.c_int
+    L.d3h_sdf_reg_backward.argtypes = [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p]
     # include/d3h_mesh.h
     L.d3h_mesh_edges_workspace_bytes.restype = C.c_int64
     L.d3h_mesh_edges_workspace_bytes.argtypes = [C.c_int64, C.c_int64]

@@ -233,6 +233,15 @@ inline void launch_k_dep(void (*kernel)(KArgs...), unsigned grid, unsigned block
 #endif
   cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
 }
+// Bits b0 .. b0 + 31 of a per-vertex bitmap as one word (the run-length scans: d3h_scan.cu, d3h_sdf_reg.cu); b0 may start
+// up to 31 bits before the first vertex (lanes outside the mask) and the upper bits may come from the word behind the
+// last vertex (allocated, never in a mask)
+__device__ __forceinline__ unsigned sign_window(const unsigned* __restrict__ occ_bits, int64_t b0) {
+  const int64_t i = b0 >> 5;
+  const unsigned lo = i >= 0 ? __ldg(occ_bits + i) : 0u, hi = __ldg(occ_bits + i + 1);
+  return __funnelshift_r(lo, hi, (unsigned)b0 & 31u);
+}
+
 d3h_counts* mapped_counts_pointer(d3h_counts* host);
 bool profiling_enabled();
 

@@ -427,14 +427,7 @@ edge_scan_pipe_kernel(const FwdBlock* __restrict__ blk, const unsigned* __restri
 //
 // The entries that found something (the surface: a few per cent) are expanded by the whole warp, lane l = lane l of the
 // entry, eight entries at a time so that the loads of their id rows are in flight together (a lane expanding its own
-// entries one after the other makes the kernel 47 us: r02y).
-__device__ __forceinline__ unsigned sign_window(const unsigned* __restrict__ occ_bits, int64_t b0) {
-  // bits b0 .. b0 + 31 of the sign bitmap; b0 may start up to 31 bits before the first vertex (lanes outside the mask)
-  // and the upper bits may come from the word behind the last vertex (allocated, never in a mask)
-  const int64_t i = b0 >> 5;
-  const unsigned lo = i >= 0 ? __ldg(occ_bits + i) : 0u, hi = __ldg(occ_bits + i + 1);
-  return __funnelshift_r(lo, hi, (unsigned)b0 & 31u);
-}
+// entries one after the other makes the kernel 47 us: r02y).  (sign_window: d3h_internal.cuh)
 __device__ __forceinline__ int64_t shfl_i64(int64_t v, int src) {
   return (int64_t)__shfl_sync(0xffffffffu, (unsigned)(v & 0xffffffffll), src) |
          ((int64_t)__shfl_sync(0xffffffffu, (unsigned)(v >> 32), src) << 32);
@@ -1194,3 +1187,8 @@ void launch_edge_scan(const d3h_forward_args& a, const Workspace& ws, cudaStream
 }
 
 }  // namespace d3h
+
+// The SDF sign-change regulariser reads the same run-length tables with the same sign windows: its kernels and entry
+// points are compiled in this translation unit, so the library and its CPU emulation (tests/emu) build them from their
+// existing source lists.
+#include "d3h_sdf_reg.cu"

@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define D3H_VERSION 500 /* 0.5.0: d3h_forward_args grew (edge_rows, edge_runs, tet_runs) */
+#define D3H_VERSION 501 /* 0.5.1: d3h_sdf_reg_* */
 
 enum {
   D3H_OK = 0,
@@ -335,6 +335,28 @@ int d3h_classify_range(const d3h_forward_args* args, d3h_tet_record* records_out
                        d3h_counts* counts_dev_out, d3h_stream_t stream);
 int d3h_extract_from_records(const d3h_forward_args* args, const d3h_tet_record* records, int64_t n_tri_tets,
                              int64_t n_quad_tets, d3h_stream_t stream);
+
+/* ---- SDF sign-change regulariser (compute_sdf_reg_loss, hmsdf.py:162-170) --------------------------------------------
+ * Over the distinct edges (a, b) of a grid, given as ONE of the two static tables of the edge scan above (edge_runs +
+ * edge_run_chunk, or edge_rows + edge_row_off, same layouts as in d3h_forward_args; the other pair NULL), an edge is
+ * selected when sign(sdf[a]) != sign(sdf[b]) with the three-valued sign (0 differs from both signs; +0.0 and -0.0 do
+ * not differ; an edge to itself is never selected).  With M selected edges:
+ *     loss = mean_e BCE(sdf[a], [sdf[b] > 0]) + mean_e BCE(sdf[b], [sdf[a] > 0]),  BCE(x, t) = (1 - t) x - log_sigmoid(x)
+ * NaN when M == 0 (the mean of an empty selection) or when sdf holds a NaN anywhere.  ±inf is not handled specially.
+ * The loss is summed in float64 in a fixed order: the same inputs give the same bits on every run.
+ * workspace: d3h_sdf_reg_workspace_bytes(N, n_edge_runs) bytes (n_edge_runs = 0 with the rows form), 16-byte aligned;
+ * the forward call leaves the sign bitmaps and M there for the backward call, which must use the same workspace, sdf
+ * and tables.  Both calls are asynchronous on `stream` and never wait for the device. */
+int64_t d3h_sdf_reg_workspace_bytes(int64_t n_grid, int64_t n_entries);
+/* *loss (one float, device memory) */
+int d3h_sdf_reg_forward(const float* sdf, int64_t n_grid, const int32_t* edge_runs, const int32_t* edge_run_chunk,
+                        int64_t n_edge_runs, const int32_t* edge_rows, const int32_t* edge_row_off, void* workspace,
+                        int64_t workspace_bytes, float* loss, d3h_stream_t stream);
+/* g_sdf[a] += g (sigmoid(sdf[a]) - [sdf[b] > 0]) / M and g_sdf[b] += g (sigmoid(sdf[b]) - [sdf[a] > 0]) / M over the
+ * selected edges; g = *g_loss (device memory), M from the workspace.  g_sdf (N) ACCUMULATES (zero it first). */
+int d3h_sdf_reg_backward(const float* sdf, int64_t n_grid, const int32_t* edge_runs, const int32_t* edge_run_chunk,
+                         int64_t n_edge_runs, const int32_t* edge_rows, const int32_t* edge_row_off, const float* g_loss,
+                         void* workspace, int64_t workspace_bytes, float* g_sdf, d3h_stream_t stream);
 
 /* ---- diagnostics (no counterpart in the reference) ------------------------------------------------------------- */
 /* Per-kernel device time: when enabled, every kernel launch of this library is bracketed by cudaEventRecord on the
